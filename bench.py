@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the MH-PPO hot path on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 Metric (BASELINE.json): agent-steps/sec of env.step.  A "step" is one env.step over the whole batch
 of synthetic envs held by a GPU.  Default workload = the configuration the north-star target is
@@ -19,6 +19,10 @@ quoted on: Env_hybrid_multi_coop_scalable, nb_car=4 / nb_ped=3 / nb_lines=2, 262
            box's host cores on a bounded sample of the same workload.
 --impl reference: the reference's own CPU path.  The reference is pure Python and cannot travel to
 the GPU box; the arm times the pinned C restatement (oracle port) with all host threads.
+--dump-outputs DIR: after the timed region, what the last timed env.step returned (env_step_*.npy) and, when the PPO
+section runs, what its last timed iteration left to the caller: rollout buffers and updated networks (ppo_*.npy); a
+fixed, seeded sample of the envs (DUMP_ENVS), float32 / float64, at most 64 MB in all.  The inputs are seeded, so two
+builds run with the same arguments can be compared array for array.
 """
 import argparse
 import json
@@ -30,6 +34,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree (it may be read-only)
 
 WORKLOADS = {
     # name: (variant, nb_car, nb_ped, nb_lines, envs per GPU)
@@ -128,6 +133,31 @@ def synthetic_actions_np(n_envs, A, seed=0):
             row.append(a)
         acts.append(row)
     return acts
+
+
+DUMP_ENVS = {"env_step": 32768, "ppo": 1024}   # envs sampled into --dump-outputs (16.8 + 25.5 MB at the default sizes)
+DUMP_LIMIT = 64 << 20
+_dumped_bytes = 0
+
+
+def dump_envs(n_envs, k):
+    """Ascending indices of a fixed, seeded sample of k of the n_envs envs (all of them when n_envs <= k)."""
+    import numpy as np
+    return np.arange(n_envs) if n_envs <= k else np.sort(np.random.default_rng(0).choice(n_envs, k, replace=False))
+
+
+def write_dump(out_dir, arrays):
+    """--dump-outputs: each tensor of `arrays` to out_dir/<name>.npy; float64 stays float64, everything else is float32."""
+    import numpy as np
+    global _dumped_bytes
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        a = a if a.dtype == np.float64 else a.astype(np.float32)
+        _dumped_bytes += a.nbytes
+        if _dumped_bytes > DUMP_LIMIT:
+            raise RuntimeError("--dump-outputs would exceed %d MB (at %s.npy)" % (DUMP_LIMIT >> 20, name))
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def cpu_port_run(variant, nb_car, nb_ped, nb_lines, n_envs, warmup, steps, threads=0, min_seconds=5.0, max_rounds=64):
@@ -233,9 +263,10 @@ def bind_to_gpu_numa_node(torch, local):
         return {"numa_node": None, "note": type(e).__name__}
 
 
-def run_ppo(mh, torch, dist, world, rank, dev, n_envs, iters, warm=2, wl=("coop_scalable", 4, 3, 2)):
+def run_ppo(mh, torch, dist, world, rank, dev, n_envs, iters, warm=2, wl=("coop_scalable", 4, 3, 2), dump_dir=None):
     """PPO samples/s (BASELINE.json metric, second half): one iteration = one 80-step episode in every env
-    (Env_rollout.iterations_rand) + reward-to-go + 10 x (cross, wait) + 10 x choice update epochs (Algo_PPO.train)."""
+    (Env_rollout.iterations_rand) + reward-to-go + 10 x (cross, wait) + 10 x choice update epochs (Algo_PPO.train).
+    dump_dir: rank 0 writes the last iteration's rollout buffers (sampled envs) and the six updated networks there."""
     variant, nb_car, nb_ped, nb_lines = wl
     env = mh.VecCrosswalkEnv(variant, n_envs, nb_car=nb_car, nb_ped=nb_ped, nb_lines=nb_lines, seed=1234, env_id0=rank * n_envs, device=dev)
     torch.manual_seed(0)
@@ -264,6 +295,19 @@ def run_ppo(mh, torch, dist, world, rank, dev, n_envs, iters, warm=2, wl=("coop_
         t_roll += e0.elapsed_time(e1); t_upd += e1.elapsed_time(e2)
         samples += sum(r.counts())
     launches = mh.launch_count() - n0
+    if dump_dir and rank == 0:
+        idx = torch.as_tensor(dump_envs(n_envs, DUMP_ENVS["ppo"]), device=dev)
+        T, Cn = r.T, r.C
+        # sample s = (t*C + car)*N + env of the [S] buffers, m = car*N + env of the [M] ones
+        out = {"ppo_" + k: getattr(r, k).view(*getattr(r, k).shape[:-1], T, Cn, n_envs)[..., idx]
+               for k in ("obs_c", "act", "logp", "rew", "rl", "rtg", "V")}
+        out.update({"ppo_" + k: getattr(r, k).view(*getattr(r, k).shape[:-1], Cn, n_envs)[..., idx]
+                    for k in ("obs_d", "act_d", "logp_d", "rew_d", "V_d")})
+        out.update(ppo_route=r.route[:, idx], ppo_exist=r.exist[:, idx])
+        # the networks as state_dict() hands them out (the reference's layout, not the kernels' padded one), concatenated
+        out.update({"ppo_%s_%s_params" % (kind, name): torch.cat([v.reshape(-1) for v in net.state_dict().values()])
+                    for name, kind, net in algo._nets()})
+        write_dump(dump_dir, out)
     # useful flops of the policy networks (SURVEY.md 8d): forward 2*(D*32 + 32*64 + 64*32 + 32*out), backward = 2 x forward
     fwd = lambda D, out: 2.0 * (D * 32 + 32 * 64 + 64 * 32 + 32 * out)
     n_c, n_w, n_d = [float(x) for x in r.counts()]
@@ -365,10 +409,14 @@ def main():
     ap.add_argument("--ppo-envs", type=int, default=131072, help="envs per GPU of the PPO samples/s section (0 = skip)")
     ap.add_argument("--ppo-iters", type=int, default=2)
     ap.add_argument("--row-major-actions", action="store_true", help="device-resident actions as a contiguous [N, A] tensor (gym layout)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step (and of the last PPO iteration) "
+                                                          "as DIR/<name>.npy, for comparing two builds")
     args = ap.parse_args()
     wl = list(WORKLOADS[args.workload])
     if args.envs:
         wl[4] = args.envs
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the GPU path (--impl ours)")
     if args.impl == "reference":
         return run_reference(args, wl)
     variant, nb_car, nb_ped, nb_lines, n_envs = wl
@@ -430,13 +478,20 @@ def main():
         if flush is not None:
             flush.zero_()
         ev[t][0].record()
-        env.step(pick(acts, W + t))
+        last = env.step(pick(acts, W + t))
         ev[t][1].record()
     barrier()
     wall = time.perf_counter() - wall0
     launches = mhppo_b200.launch_count() - n0
     step_ms = [a.elapsed_time(b) for a, b in ev]
     dev_ms = sum(step_ms)
+    if args.dump_outputs and rank == 0:          # before the end-to-end region steps the same envs further
+        obs, rew, done, trunc, _ = last
+        idx = torch.as_tensor(dump_envs(n_envs, DUMP_ENVS["env_step"]), device=dev)
+        out = {"env_step_obs_" + k: v[idx] for k, v in obs.items()}
+        out.update(env_step_rewards=rew[idx], env_step_done=done[idx], env_step_truncated=trunc[idx],
+                   env_step_reward_light=env.reward_light[idx], env_step_terminal_obs=env.terminal_obs[idx])
+        write_dump(args.dump_outputs, out)
 
     # ---- end-to-end region: host buffers through the reference-facing call -------------------------
     Ke = max(8, min(K, 40))
@@ -459,14 +514,15 @@ def main():
     st = env.get_state()
     active = float((st["env_i"][:, 1] + st["env_i"][:, 2]).float().mean().item())
     flushed = flush is not None
-    del st, env, flush, acts, act_h, obs_h
+    del st, env, last, flush, acts, act_h, obs_h
     torch.cuda.empty_cache()
     ppo = None
     if args.ppo_envs > 0 and args.ppo_iters > 0:
         if args.workload == "scalable_432":
-            ppo = run_ppo(mhppo_b200, torch, dist, world, rank, dev, args.ppo_envs, args.ppo_iters)
+            ppo = run_ppo(mhppo_b200, torch, dist, world, rank, dev, args.ppo_envs, args.ppo_iters, dump_dir=args.dump_outputs)
         elif variant in ("coop", "naif", "stop"):       # the older drivers' PPO on their own env class, at the workload's env count
-            ppo = run_ppo(mhppo_b200, torch, dist, world, rank, dev, n_envs, max(args.ppo_iters, 5), warm=3, wl=(variant, nb_car, nb_ped, nb_lines))
+            ppo = run_ppo(mhppo_b200, torch, dist, world, rank, dev, n_envs, max(args.ppo_iters, 5), warm=3, wl=(variant, nb_car, nb_ped, nb_lines),
+                          dump_dir=args.dump_outputs)
     clocks = sampler.stop()        # sampled every 200 ms from the start of the device-timed region to the end of the PPO section
     t_dev = torch.tensor([dev_ms, e2e_s, active], dtype=torch.float64, device=dev)
     if world > 1:
