@@ -241,6 +241,25 @@ int mhppo_ppo_grad_dev(int32_t n_in, int32_t head, const float *x_dev, int32_t D
                        int64_t CN, const float *net_dev, const float *act_dev, const float *logp_old_dev, const float *rtg_dev,
                        const float *V_dev, const double *adv_stats_dev, float inv_n, float f0, float f1, float *grad_dev,
                        double *loss_dev, void *workspace_dev, void *stream);
+/* mhppo_ppo_grad_dev plus an entropy bonus for the categorical choice actor (an option; the reference's loss has none):
+ * loss -= ent_coef * inv_n * sum_s H(pi(.|s)), H = -sum_k p_k log p_k over the two-way softmax, log p_k formed as log-softmax
+ * (finite for saturated logits).  ent_coef == 0 runs exactly the kernel of mhppo_ppo_grad_dev (bit-identical results).
+ * MHPPO_EINVAL for a non-finite ent_coef or a non-zero one with head != 2 (the Gaussian heads have a fixed variance: their
+ * entropy is a constant without gradient). */
+int mhppo_ppo_grad_ent(int32_t n_in, int32_t head, const float *x_dev, int32_t D, int64_t S, const int32_t *idx_dev, int64_t K,
+                       int64_t CN, const float *net_dev, const float *act_dev, const float *logp_old_dev, const float *rtg_dev,
+                       const float *V_dev, const double *adv_stats_dev, float inv_n, float f0, float f1, float ent_coef,
+                       float *grad_dev, double *loss_dev, void *workspace_dev, void *stream);
+/* GAE(gamma, lambda) returns of the cross / wait buffers (an option; the reference's estimator is mhppo_returns, i.e. lambda = 1
+ * with the critic recomputed every epoch).  Per column m of route_dev int8 [CN] (0 cross, 1 wait, -1 absent) over
+ * t = T-1 .. 0 with V(s_T) = 0, R_T = 0, in fp64:  R_t = r_t + gamma ((1 - lambda) V(s_{t+1}) + lambda R_{t+1}),
+ * ret_t = (float)R_t, A_t = ret_t - V(s_t) (fp32, as the actor forms it).  V_dev: V_old of the update (mhppo_value_stats of
+ * each buffer's critic on its selection).  Absent columns get ret = 0 and are not read.  stats6_dev: (sum A, sum A^2, n) of
+ * route 0, then of route 1, in a fixed summation order (bitwise repeatable); +0 / +3 are adv_stats_dev of the cross / wait
+ * actor.  At lambda = 1 ret equals mhppo_returns' rtg bit for bit.  workspace_dev: 196 608 bytes (any update workspace of
+ * mhppo_update_workspace_bytes is larger).  MHPPO_EINVAL for null pointers, T < 1, CN < 1, gamma or lambda outside [0, 1]. */
+int mhppo_gae(const float *rew_dev, const float *V_dev, const int8_t *route_dev, int32_t T, int64_t CN, double gamma, double lambda,
+              float *ret_dev, double *stats6_dev, void *workspace_dev, void *stream);
 /* critic pass of one epoch in a single kernel: ppo_grad with head 0 that also returns V = critic(s) (PY:785) and the
  * advantage statistics (sum A, sum A^2, n) of A = rtg - V, so an epoch is critic_grad_stats -> [all-reduce stats] ->
  * ppo_grad (actor) -> [all-reduce grads] -> adam, adam; V and the statistics are those of the critic before its step,

@@ -112,7 +112,8 @@ static int launch_grad(int head, const SampleSet &ss, const float *net, const Lo
     // (the tensor-core kernel stages exactly the 13 features of the cross / wait nets; a wider 16-padded input takes the FFMA kernel)
     if (KP == 16 && ss.D <= 13 && head != 2 && use_tc(false)) return launch_grad_tc(head, ss, net, la, w, s);
     const size_t sm = smem_grad<KP>();
-    if (head == 0) { SET_SMEM((k_ppo_grad<KP, 0>), sm); k_ppo_grad<KP, 0><<<kGradGrid, kMlpBlock, sm, s>>>(ss, net, la, w.gpartial, w.lpartial); }
+    if (head == 2 && la.ent_coef != 0.f) { SET_SMEM((k_ppo_grad<KP, 2, true>), sm); k_ppo_grad<KP, 2, true><<<kGradGrid, kMlpBlock, sm, s>>>(ss, net, la, w.gpartial, w.lpartial); }
+    else if (head == 0) { SET_SMEM((k_ppo_grad<KP, 0>), sm); k_ppo_grad<KP, 0><<<kGradGrid, kMlpBlock, sm, s>>>(ss, net, la, w.gpartial, w.lpartial); }
     else if (head == 1) { SET_SMEM((k_ppo_grad<KP, 1>), sm); k_ppo_grad<KP, 1><<<kGradGrid, kMlpBlock, sm, s>>>(ss, net, la, w.gpartial, w.lpartial); }
     else { SET_SMEM((k_ppo_grad<KP, 2>), sm); k_ppo_grad<KP, 2><<<kGradGrid, kMlpBlock, sm, s>>>(ss, net, la, w.gpartial, w.lpartial); }
     api_count_launch();
@@ -352,7 +353,7 @@ int mhppo_value_stats(int32_t n_in, const float *x, int32_t D, int64_t S, const 
 static int ppo_grad_impl(int32_t n_in, int32_t head, const float *x, int32_t D, int64_t S, const int32_t *idx, int64_t K, int64_t CN,
                          const float *net, const float *act, const float *logp_old, const float *rtg, const float *V, float adv_mean,
                          float adv_inv_std, float inv_n, float f0, float f1, float *grad, double *loss, float *V_out, double *stats3,
-                         const double *adv_stats_dev, void *workspace, void *stream) {
+                         const double *adv_stats_dev, void *workspace, void *stream, float ent_coef = 0.f) {
     if (!x || !net || !rtg || !grad || !loss || !workspace) return api_fail(MHPPO_EINVAL, "null argument");
     if (head < 0 || head > 2) return api_fail(MHPPO_EINVAL, "head must be 0, 1 or 2");
     if (head != 0 && (!act || !logp_old || !V)) return api_fail(MHPPO_EINVAL, "actor heads need act, logp_old and V");
@@ -363,7 +364,7 @@ static int ppo_grad_impl(int32_t n_in, int32_t head, const float *x, int32_t D, 
     const Workspace w = carve(workspace, kp);
     LossArgs la; la.act = act; la.logp_old = logp_old; la.rtg = rtg; la.V = V; la.adv_mean = adv_mean; la.adv_inv_std = adv_inv_std;
     la.inv_n = inv_n; la.f0 = f0; la.f1 = f1; la.V_out = V_out; la.spartial = stats3 ? w.spartial : nullptr;
-    la.head = g_head; la.stats_dev = adv_stats_dev;
+    la.head = g_head; la.stats_dev = adv_stats_dev; la.ent_coef = ent_coef;
     cudaStream_t s = (cudaStream_t)stream;
     int rc = (kp == 16) ? launch_grad<16>(head, ss, net, la, w, s) : ((kp == 32) ? launch_grad<32>(head, ss, net, la, w, s) : launch_grad<56>(head, ss, net, la, w, s));
     if (rc) return rc;
@@ -387,6 +388,36 @@ int mhppo_ppo_grad_dev(int32_t n_in, int32_t head, const float *x, int32_t D, in
     if (!adv_stats_dev) return api_fail(MHPPO_EINVAL, "null argument");
     return ppo_grad_impl(n_in, head, x, D, S, idx, K, CN, net, act, logp_old, rtg, V, 0.f, 0.f, inv_n, f0, f1, grad, loss, nullptr, nullptr,
                          adv_stats_dev, workspace, stream);
+}
+
+int mhppo_ppo_grad_ent(int32_t n_in, int32_t head, const float *x, int32_t D, int64_t S, const int32_t *idx, int64_t K, int64_t CN,
+                       const float *net, const float *act, const float *logp_old, const float *rtg, const float *V,
+                       const double *adv_stats_dev, float inv_n, float f0, float f1, float ent_coef, float *grad, double *loss,
+                       void *workspace, void *stream) {
+    if (!adv_stats_dev) return api_fail(MHPPO_EINVAL, "null argument");
+    if (!std::isfinite(ent_coef)) return api_fail(MHPPO_EINVAL, "ent_coef must be finite");
+    if (ent_coef != 0.f && head != 2) return api_fail(MHPPO_EINVAL, "the entropy bonus needs head 2 (categorical choice actor)");
+    return ppo_grad_impl(n_in, head, x, D, S, idx, K, CN, net, act, logp_old, rtg, V, 0.f, 0.f, inv_n, f0, f1, grad, loss, nullptr, nullptr,
+                         adv_stats_dev, workspace, stream, ent_coef);
+}
+
+int mhppo_gae(const float *rew, const float *V, const int8_t *route, int32_t T, int64_t CN, double gamma, double lambda, float *ret,
+              double *stats6, void *workspace, void *stream) {
+    if (!rew || !V || !route || !ret || !stats6 || !workspace) return api_fail(MHPPO_EINVAL, "null argument");
+    if (T < 1 || CN < 1) return api_fail(MHPPO_EINVAL, "T and CN must be >= 1");
+    if (!(gamma >= 0.0 && gamma <= 1.0) || !(lambda >= 0.0 && lambda <= 1.0)) return api_fail(MHPPO_EINVAL, "gamma and lambda must lie in [0, 1]");
+    const int64_t blocks = (CN + kGaeBlock - 1) / kGaeBlock;
+    const int cap = 8 * sm_count() < kGaeGridMax ? 8 * sm_count() : kGaeGridMax;
+    const int grid = blocks < cap ? (int)blocks : cap;
+    double *partial = (double *)workspace;
+    cudaStream_t s = (cudaStream_t)stream;
+    k_gae<<<grid, kGaeBlock, 0, s>>>(rew, V, route, T, CN, gamma, lambda, ret, partial);
+    api_count_launch();
+    int rc = ck(cudaGetLastError(), "k_gae");
+    if (rc) return rc;
+    k_reduce_gae<<<1, 192, 0, s>>>(partial, grid, stats6);
+    api_count_launch();
+    return ck(cudaGetLastError(), "k_reduce_gae");
 }
 
 int mhppo_critic_grad_stats(int32_t n_in, const float *x, int32_t D, int64_t S, const int32_t *idx, int64_t K, int64_t CN,

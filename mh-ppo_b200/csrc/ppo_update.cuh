@@ -94,6 +94,7 @@ struct LossArgs {
     HeadCfg head;                              // Gaussian head (HEAD == 1)
     const double *stats_dev;                   // actor heads, optional: (sum A, sum A^2, n) of the whole (all-rank) batch in device
                                                //   memory; adv_mean / adv_inv_std are then derived in the kernel (no host round trip)
+    float ent_coef;                            // choice only: entropy bonus c; read only by the k_ppo_grad<KP, 2, true> instances
 };
 
 // advantage normalisation of PY:787 from the partial sums: mean, 1 / (unbiased std + 1e-10) (Algo_PPO.combine_stats)
@@ -244,8 +245,10 @@ __device__ __forceinline__ LossIn load_loss_in(const LossArgs &la, int64_t s) {
     if (HEAD == 1) in.act = la.act[s];
     return in;
 }
-template <int HEAD>
+// ENT (HEAD == 2 only): adds the entropy bonus -c * inv_n * H(pi(.|s)) to the loss; ENT = false is the reference's loss
+template <int HEAD, bool ENT = false>
 __device__ __forceinline__ void ppo_loss(const LossArgs &la, int64_t s, const LossIn &in, float4 o, float (&dz)[OP], LossAcc &acc) {
+    static_assert(!ENT || HEAD == 2, "the entropy bonus exists for the categorical head only");
     if (HEAD == 0) {                                           // critic_loss = MSE(V, rtg), PY:808-809
         const float e = o.x - in.rtg;
         acc.loss += (double)e * (double)e * (double)la.inv_n;
@@ -286,6 +289,14 @@ __device__ __forceinline__ void ppo_loss(const LossArgs &la, int64_t s, const Lo
         // softmax backward: dz_a = p_a * (dp_a - sum_b p_b dp_b)
         const float dot = p0 * dp0 + p1 * dp1;
         dz[0] = p0 * (dp0 - dot); dz[1] = p1 * (dp1 - dot);
+        if (ENT) {
+            // H = -sum_k p_k log p_k with log p_k = z_k - m - log(e0 + e1): finite for logits any distance apart (p_k = 0 has
+            // log p_k = z_k - m, so p_k log p_k = 0); dLoss/dz_k = c * inv_n * p_k * (log p_k + H)
+            const float lse = logf(e0 + e1), lp0 = (o.x - m) - lse, lp1 = (o.y - m) - lse;
+            const float H = -(p0 * lp0 + p1 * lp1), ci = la.ent_coef * la.inv_n;
+            acc.loss -= (double)la.ent_coef * (double)la.inv_n * (double)H;
+            dz[0] += ci * p0 * (lp0 + H); dz[1] += ci * p1 * (lp1 + H);
+        }
     }
 }
 
@@ -388,7 +399,7 @@ struct WgradAcc {
 // Per tile: [thread = R samples] forward + loss + dz; then, layer by layer from the top, [register tiles] weight gradient from
 // (input activation, delta) and [thread = R samples] backward-data which overwrites the activation with its delta.
 constexpr int kTeams = 1;
-template <int KP, int HEAD>
+template <int KP, int HEAD, bool ENT = false>
 __global__ void __launch_bounds__(kMlpBlock, 1) k_ppo_grad(SampleSet ss, const float *__restrict__ net, LossArgs la,
                                                            float *__restrict__ gpartial /* [grid][net_params] */,
                                                            double *__restrict__ lpartial /* [grid] */) {
@@ -444,7 +455,7 @@ __global__ void __launch_bounds__(kMlpBlock, 1) k_ppo_grad(SampleSet ss, const f
         for (int r = 0; r < R; ++r) {
             float *row = my + r * RS;
             float dz[OP] = {0.f, 0.f, 0.f, 0.f};
-            if (sel[r]) ppo_loss<HEAD>(la, sidx[r], load_loss_in<HEAD>(la, sidx[r]), ld4(row + G::D4), dz, acc);
+            if (sel[r]) ppo_loss<HEAD, ENT>(la, sidx[r], load_loss_in<HEAD>(la, sidx[r]), ld4(row + G::D4), dz, acc);
             // an unselected row has x = 0 but its activations are relu(bias) != 0: its dz = 0 keeps every gradient term zero
             st4(row + G::D4, make_float4(dz[0], dz[1], dz[2], dz[3]));
         }
@@ -497,6 +508,63 @@ __global__ void k_reduce_scalars(const double *__restrict__ partial, int nblocks
     double acc = 0.0;
     for (int b = 0; b < nblocks; ++b) acc += partial[(size_t)b * width + j];
     out[j] = acc;
+}
+
+// ---- GAE(gamma, lambda) returns of the cross / wait buffers (an option; the reference's estimator is k_returns) ----------
+// One thread per (car, env) column m, reverse scan over t with V(s_T) = 0 and R_T = 0 (the episode ends at step T-1):
+//   R_t = r_t + gamma * ((1 - lambda) * V_old(s_{t+1}) + lambda * R_{t+1}),   ret_t = (float)R_t,   A_t = ret_t - V_old(s_t)
+// so A_t = sum_k (gamma lambda)^k delta_{t+k}.  The recursion is fp64 without contraction (__dmul_rn / __dadd_rn): at lambda = 1
+// it is r_t + gamma * R_{t+1}, the operations of k_returns, and ret equals that reward-to-go bit for bit.  A is formed in fp32
+// as the actor kernel forms it (rtg - V).  Columns with route -1 (car absent) are written +0 and read nothing.  Each CTA writes
+// fp64 partials (sum A, sum A^2, n) of route 0 then route 1; k_reduce_gae adds them in a fixed order (no atomics).
+// Every access of a step is coalesced over m; the kGaeUnroll loads of a batch of steps are independent (memory parallelism).
+constexpr int kGaeBlock = 256, kGaeGridMax = 4096, kGaeUnroll = 8;    // grid: min(columns / 256, 8 per SM, 4096 = workspace rows)
+__global__ void __launch_bounds__(kGaeBlock) k_gae(const float *__restrict__ rew, const float *__restrict__ V,
+                                                   const int8_t *__restrict__ route, int T, int64_t CN, double gamma, double lambda,
+                                                   float *__restrict__ ret, double *__restrict__ partial /* [grid][6] */) {
+    __shared__ double red[kGaeBlock / 32];
+    double st[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+    const double oml = 1.0 - lambda;
+    for (int64_t m = (int64_t)blockIdx.x * kGaeBlock + threadIdx.x; m < CN; m += (int64_t)gridDim.x * kGaeBlock) {
+        const int r = route[m];
+        const bool on = r >= 0;         // an absent column runs the same scan on zeros (no divergence in the warp): R = +0 throughout
+        double R = 0.0, Vn = 0.0, sA = 0.0, sAA = 0.0;
+        for (int t0 = T - 1; t0 >= 0; t0 -= kGaeUnroll) {
+            float rw[kGaeUnroll], v[kGaeUnroll];
+#pragma unroll
+            for (int u = 0; u < kGaeUnroll; ++u) {
+                const int64_t s = (int64_t)(t0 - u) * CN + m;
+                rw[u] = (on && t0 - u >= 0) ? rew[s] : 0.f;
+                v[u] = (on && t0 - u >= 0) ? V[s] : 0.f;
+            }
+#pragma unroll
+            for (int u = 0; u < kGaeUnroll; ++u) {
+                if (t0 - u < 0) break;
+                R = __dadd_rn((double)rw[u], __dmul_rn(gamma, __dadd_rn(__dmul_rn(oml, Vn), __dmul_rn(lambda, R))));
+                const float Rf = (float)R;
+                ret[(int64_t)(t0 - u) * CN + m] = Rf;
+                const double A = (double)(Rf - v[u]);
+                sA += A; sAA += A * A;
+                Vn = (double)v[u];
+            }
+        }
+        if (r == 0) { st[0] += sA; st[1] += sAA; st[2] += (double)T; }
+        else if (r == 1) { st[3] += sA; st[4] += sAA; st[5] += (double)T; }
+    }
+#pragma unroll
+    for (int j = 0; j < 6; ++j) {
+        const double v = team_sum(st[j], red, threadIdx.x, kGaeBlock, 0);
+        if (threadIdx.x == 0) partial[(size_t)blockIdx.x * 6 + j] = v;
+    }
+}
+// fixed-order sum of the k_gae partials [n][6]: warp j adds column j (lane l takes rows l, l + 32, ..., then a shuffle tree),
+// so the up to kGaeGridMax rows cost a few independent loads per lane instead of one serial chain
+__global__ void __launch_bounds__(192) k_reduce_gae(const double *__restrict__ partial, int n, double *__restrict__ out) {
+    const int j = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    double acc = 0.0;
+    for (int b = lane; b < n; b += 32) acc += partial[(size_t)b * 6 + j];
+    for (int o = 16; o > 0; o >>= 1) acc += __shfl_down_sync(0xffffffffu, acc, o);
+    if (lane == 0) out[j] = acc;
 }
 
 // ---- 6. Adam (torch.optim.Adam defaults, PY:719-724): p -= step_size * m / (sqrt(v) * inv_sqrt_bc2 + eps) ----

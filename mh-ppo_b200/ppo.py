@@ -3,6 +3,11 @@ scalable env class: same constructor (`Algo_PPO(policy_class, env, **hyperparame
 and six Adam optimisers, same update rule (clipped surrogate 0.8/1.2, no entropy term, MSE critic, 10 full-batch
 epochs per net per iteration, advantages = reward-to-go - V normalised with the unbiased std).
 
+Two options beyond the reference, both off by default (DESIGN.md §4 "GAE and entropy options"):
+  gae_lambda=None   a number in [0, 1]: the cross / wait nets train on GAE(gamma, lambda) returns and advantages, formed
+                    once per update from the critics before the update (Env_rollout.gae); the choice net is unchanged
+  entropy_coef=0.0  c > 0: the choice actor's loss gets the entropy bonus -c * mean_s H(pi(.|s))
+
 One iteration = one 80-step episode in every env of the vectorised env.  Multi-GPU: one process per GPU, envs
 sharded per rank; the only collectives are the all-reduce of the three advantage statistics and of the flat
 gradient buffers (NCCL through torch.distributed), so an R-rank run performs the same update as one rank
@@ -10,6 +15,7 @@ holding all envs (SURVEY.md 8e).
 """
 import ctypes as C
 import math
+import numbers
 import os
 
 import numpy as np
@@ -56,6 +62,7 @@ def allreduce_sum_(t):
 class Algo_PPO:
     def __init__(self, policy_class, env, **hyperparameters):
         self._init_hyperparameters(hyperparameters)
+        self._check_options()
         self.env = env
         self.max_steps = env.max_episode
         dev = env.device
@@ -115,8 +122,20 @@ class Algo_PPO:
         self.num_algo, self.total_loop, self.batch_size, self.gamma = 1, 0, 2048, 0.99
         self.critic_lr, self.actor_lr, self.critic_d_lr, self.actor_d_lr = 1e-3, 3e-4, 1e-3, 3e-4
         self.num_states_c, self.num_states_d, self.num_actions, self.mean, self.std, self.dt = 13, None, 1, -1.0, 3.0, 0.3
+        self.gae_lambda, self.entropy_coef = None, 0.0                     # options beyond the reference (module docstring)
         for k, v in hyperparameters.items():
             setattr(self, k, v)
+
+    def _check_options(self):
+        real = lambda v: isinstance(v, numbers.Real) and not isinstance(v, bool)
+        lam, c = self.gae_lambda, self.entropy_coef
+        if lam is not None:
+            if not (real(lam) and 0.0 <= float(lam) <= 1.0):
+                raise ValueError("gae_lambda must be None or a number in [0, 1], got %r" % (lam,))
+            if not (real(self.gamma) and 0.0 <= float(self.gamma) <= 1.0):
+                raise ValueError("GAE needs gamma in [0, 1], got %r" % (self.gamma,))
+        if not (real(c) and math.isfinite(float(c)) and float(c) >= 0.0):
+            raise ValueError("entropy_coef must be a finite number >= 0, got %r" % (c,))
 
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.env.device).cuda_stream)
@@ -150,6 +169,17 @@ class Algo_PPO:
         n = self._global_count(want, K * (r.S // r.M))             # sample slots: S = T * M, M = C * N columns
         if n < 1:
             return False                                     # PY:869/874: the net is skipped when its buffer is empty
+        if self.gae_lambda is not None:
+            # GAE: fixed targets ret and advantages ret - V_old of this update; the critic pass must not overwrite V_old
+            stats = self._gae_stats()
+            check(L.mhppo_ppo_grad(13, 0, r.obs_c.data_ptr(), 13, r.S, idx.data_ptr(), K, r.M, critic.flat.data_ptr(), None, None,
+                                   r.ret.data_ptr(), None, 0.0, 0.0, 1.0 / n, 0.0, 0.0, critic.grad.data_ptr(), self._loss.data_ptr() + 8,
+                                   ws, st))
+            check(L.mhppo_ppo_grad_dev(13, 1, r.obs_c.data_ptr(), 13, r.S, idx.data_ptr(), K, r.M, actor.flat.data_ptr(),
+                                       r.act.data_ptr(), r.logp.data_ptr(), r.ret.data_ptr(), r.V.data_ptr(), stats.data_ptr() + 24 * want,
+                                       1.0 / n, 0.0, 0.0, actor.grad.data_ptr(), self._loss.data_ptr(), ws, st))
+            self._step_pair(actor, critic, opti_actor, opti_critic)
+            return True
         # critic pass first: its forward is V = critic(s) of PY:785, so the same kernel returns V and the advantage statistics
         check(L.mhppo_critic_grad_stats(13, r.obs_c.data_ptr(), 13, r.S, idx.data_ptr(), K, r.M, critic.flat.data_ptr(),
                                         r.rtg.data_ptr(), 1.0 / n, critic.grad.data_ptr(), self._loss.data_ptr() + 8,
@@ -160,6 +190,18 @@ class Algo_PPO:
                                    0.0, 0.0, actor.grad.data_ptr(), self._loss.data_ptr(), ws, st))
         self._step_pair(actor, critic, opti_actor, opti_critic)
         return True
+
+    def _prepare_gae(self):
+        """GAE mode, once per update before the epochs: V_old of both critics, the returns and the advantage statistics of
+        the cross and wait samples, all-reduced over the ranks once."""
+        _, stats6 = self.rollout.gae(self.critic_net_cross, self.critic_net_wait, self.gamma, self.gae_lambda,
+                                     selections=(self._selection(0), self._selection(1)), workspace=self._ws)
+        self._sel_cache["gae"] = allreduce_sum_(stats6)
+
+    def _gae_stats(self):
+        if "gae" not in self._sel_cache:                    # train_model_c called outside update() on a new rollout
+            self._prepare_gae()
+        return self._sel_cache["gae"]
 
     def _step_pair(self, actor, critic, opti_actor, opti_critic):
         """All-reduce the pair's packed gradients (one collective) and take both Adam steps in one launch (PY:810-815)."""
@@ -182,6 +224,12 @@ class Algo_PPO:
                                         r.V_d.data_ptr(), self._stats.data_ptr(), ws, st))
         allreduce_sum_(self._stats)
         f0, f1 = self._action_fractions(n)
+        if self.entropy_coef:
+            check(L.mhppo_ppo_grad_ent(D, 2, r.obs_d.data_ptr(), D, r.M, idx.data_ptr(), K, r.M, actor.flat.data_ptr(),
+                                       r.act_d.data_ptr(), r.logp_d.data_ptr(), r.rew_d.data_ptr(), r.V_d.data_ptr(), self._stats.data_ptr(),
+                                       1.0 / n, f0, f1, float(self.entropy_coef), actor.grad.data_ptr(), self._loss.data_ptr(), ws, st))
+            self._step_pair(actor, critic, opti_actor, opti_critic)
+            return True
         check(L.mhppo_ppo_grad_dev(D, 2, r.obs_d.data_ptr(), D, r.M, idx.data_ptr(), K, r.M, actor.flat.data_ptr(),
                                    r.act_d.data_ptr(), r.logp_d.data_ptr(), r.rew_d.data_ptr(), r.V_d.data_ptr(), self._stats.data_ptr(),
                                    1.0 / n, f0, f1, actor.grad.data_ptr(), self._loss.data_ptr(), ws, st))
@@ -203,7 +251,9 @@ class Algo_PPO:
         """The update half of train() (PY:866-882): 10 x (cross, wait) then 10 x choice."""
         self.rollout.value_std = self.value_std
         self.rollout._set_head(self.actor_net_cross)
-        self.rollout.futur_rewards()
+        self.rollout.futur_rewards()                    # also the choice reward rew_d, which GAE mode uses too
+        if self.gae_lambda is not None:
+            self._prepare_gae()
         for _ in range(epochs):
             self.train_model_c(self.actor_net_cross, self.critic_net_cross, self.optimizer_actor_cross, self.optimizer_critic_cross, 0)
             self.train_model_c(self.actor_net_wait, self.critic_net_wait, self.optimizer_actor_wait, self.optimizer_critic_wait, 1)

@@ -46,6 +46,7 @@ class Env_rollout:
         self.iteration = 0
         self.use_graph = True                            # replay the T-step loop as a CUDA graph (mhppo_rollout_steps)
         self.value_std = 0.5                             # exploration variance of the Gaussian head (Algo_PPO.value_std, PY:726)
+        self.ret = None                                  # GAE returns [S]: allocated by the first gae() call
 
     def _set_head(self, actor):
         """The kernels' Gaussian head = the actor's own (tanh * std + mean, PY:88-90), the noise variance of PY:726-729 and
@@ -242,6 +243,34 @@ class Env_rollout:
         check(self._L.mhppo_returns(self.rew.data_ptr(), self.rl.data_ptr(), self.T, self.M, 0.99, self.rtg.data_ptr(),
                                     self.rew_d.data_ptr(), self._stream()))
         return self.rtg, self.rew_d
+
+    def gae(self, critic_cross, critic_wait, gamma, lam, selections=None, workspace=None):
+        """GAE(gamma, lambda) returns of the cross / wait buffers, an option of Algo_PPO (the reference's estimator is
+        futur_rewards: lambda = 1 against the critic of every epoch).  Each critic evaluates V_old(s) once on the samples
+        routed to its net (mhppo_value_stats, into self.V), then one reverse scan per (car, env) column (mhppo_gae) with
+        V(s_T) = 0.  selections: the (idx, K) compacted column lists of route 0 and 1 (Algo_PPO._selection), built from
+        `route` when None.  Returns (ret [S], stats6): the regression targets and this rank's advantage statistics
+        (sum A, sum A^2, n) of the cross samples, then of the wait samples.  The buffers are allocated on the first call."""
+        L, st, dev = self._L, self._stream(), self.rew.device
+        if self.ret is None:
+            self.ret = torch.zeros(self.S, device=dev)
+            self._gae_stats = torch.zeros(9, dtype=torch.float64, device=dev)      # stats6 | scratch of mhppo_value_stats
+        if workspace is None:
+            if getattr(self, "_gae_ws", None) is None:
+                self._gae_ws = torch.zeros(L.mhppo_update_workspace_bytes(13), dtype=torch.uint8, device=dev)
+            workspace = self._gae_ws
+        if selections is None:
+            selections = []
+            for want in (0, 1):
+                sel = torch.nonzero(self.route.view(-1) == want).view(-1).to(torch.int32)
+                selections.append((sel if sel.numel() else torch.zeros(1, dtype=torch.int32, device=dev), sel.numel()))
+        ws, scratch = workspace.data_ptr(), self._gae_stats.data_ptr() + 6 * 8
+        for critic, (idx, K) in zip((critic_cross, critic_wait), selections):
+            check(L.mhppo_value_stats(13, self.obs_c.data_ptr(), 13, self.S, idx.data_ptr(), K, self.M, critic.flat.data_ptr(),
+                                      self.rew.data_ptr(), self.V.data_ptr(), scratch, ws, st))
+        check(L.mhppo_gae(self.rew.data_ptr(), self.V.data_ptr(), self.route.data_ptr(), self.T, self.M, float(gamma), float(lam),
+                          self.ret.data_ptr(), self._gae_stats.data_ptr(), ws, st))
+        return self.ret, self._gae_stats[:6]
 
     def counts(self):
         """(cross, wait, choice) sample counts of the last rollout."""
