@@ -260,6 +260,22 @@ int mhppo_ppo_grad_ent(int32_t n_in, int32_t head, const float *x_dev, int32_t D
  * mhppo_update_workspace_bytes is larger).  MHPPO_EINVAL for null pointers, T < 1, CN < 1, gamma or lambda outside [0, 1]. */
 int mhppo_gae(const float *rew_dev, const float *V_dev, const int8_t *route_dev, int32_t T, int64_t CN, double gamma, double lambda,
               float *ret_dev, double *stats6_dev, void *workspace_dev, void *stream);
+/* Minibatch plan of an update (an option, Algo_PPO(n_minibatches=B); the reference's update is full-batch, PY:866-882).
+ * In epoch e (0 .. epochs-1) the (car, env) column m = car*N + n, global env id g = cfg->env_id0 + n, goes to bucket
+ *   b = (x0 * B) >> 32,  x0 = word 0 of Philox4x32-10(counter = (e*C + car, 3 | iteration << 8, g_lo, g_hi), key = cfg->seed)
+ * (stream 3 of the policy-noise contract; iteration = the rollout that filled the buffers), so a sharded run forms the same global
+ * minibatches as one rank holding every env.  route_dev / exist_dev int8 [C][N], act_d_dev float [C*N] (choice actions 0 / 1).
+ * Outputs, per epoch, for the selections s = 0 cross (route 0), 1 wait (route 1), 2 existing cars (exist != 0):
+ *   lists_dev   int32 [epochs][3][C*N]: bucket-major column lists, ascending m within a bucket (at B = 1 the compacted lists of
+ *               torch.nonzero); bucket b of selection s is lists[e][s][offsets[e][s][b] .. offsets[e][s][b+1])
+ *   offsets_dev int64 [epochs][3][B+1]
+ *   counts_dev  int64 [epochs][5][B]: bucket sizes of the three selections, then the existing columns whose choice action is 0 / 1
+ * Integer counting sort in a fixed order (no order from atomics): repeated calls give identical outputs.  Three launches.
+ * workspace_dev: 1280 * epochs * B bytes.  MHPPO_EINVAL for null pointers, epochs < 1, B outside [1, 1024] (the per-tile
+ * histograms of five rows x B buckets live in 20 KB of shared memory), N < 1 or C*N >= 2^31. */
+int mhppo_minibatch_plan(const mhppo_rollout_cfg *cfg, const int8_t *route_dev, const int8_t *exist_dev, const float *act_d_dev,
+                         uint32_t iteration, int32_t epochs, int32_t n_minibatches, int32_t *lists_dev, int64_t *offsets_dev,
+                         int64_t *counts_dev, void *workspace_dev, void *stream);
 /* critic pass of one epoch in a single kernel: ppo_grad with head 0 that also returns V = critic(s) (PY:785) and the
  * advantage statistics (sum A, sum A^2, n) of A = rtg - V, so an epoch is critic_grad_stats -> [all-reduce stats] ->
  * ppo_grad (actor) -> [all-reduce grads] -> adam, adam; V and the statistics are those of the critic before its step,

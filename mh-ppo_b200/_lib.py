@@ -76,6 +76,7 @@ SYMBOLS = {
     "mhppo_ppo_grad_ent": (C.c_int, [C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_int64, C.c_int64]
                            + [C.c_void_p] * 6 + [C.c_float] * 4 + [C.c_void_p] * 4),
     "mhppo_gae": (C.c_int, [C.c_void_p] * 3 + [C.c_int32, C.c_int64, C.c_double, C.c_double] + [C.c_void_p] * 4),
+    "mhppo_minibatch_plan": (C.c_int, [C.POINTER(RolloutCfg)] + [C.c_void_p] * 3 + [C.c_uint32, C.c_int32, C.c_int32] + [C.c_void_p] * 5),
     "mhppo_adam2": (C.c_int, [C.c_void_p] * 4 + [C.c_int32, C.c_float, C.c_int32] + [C.c_void_p] * 4 + [C.c_int32, C.c_float, C.c_int32]
                     + [C.c_float] * 3 + [C.c_void_p]),
     "mhppo_tc_failures": (C.c_int, []),

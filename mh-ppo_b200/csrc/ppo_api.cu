@@ -420,6 +420,34 @@ int mhppo_gae(const float *rew, const float *V, const int8_t *route, int32_t T, 
     return ck(cudaGetLastError(), "k_reduce_gae");
 }
 
+int mhppo_minibatch_plan(const mhppo_rollout_cfg *cfg, const int8_t *route, const int8_t *exist, const float *act_d, uint32_t iteration,
+                         int32_t epochs, int32_t n_minibatches, int32_t *lists, int64_t *offsets, int64_t *counts, void *workspace,
+                         void *stream) {
+    if (!cfg || !route || !exist || !act_d || !lists || !offsets || !counts || !workspace) return api_fail(MHPPO_EINVAL, "null argument");
+    if (epochs < 1) return api_fail(MHPPO_EINVAL, "epochs must be >= 1");
+    if (n_minibatches < 1 || n_minibatches > kMbMaxBuckets) return api_fail(MHPPO_EINVAL, "n_minibatches must lie in [1, 1024]");
+    const RolloutDims d = dims_of(cfg);
+    const int64_t M = (int64_t)d.C * d.N;
+    if (d.N < 1 || d.C < 1 || M > 0x7fffffff) return api_fail(MHPPO_EINVAL, "bad rollout dimensions");
+    MbPlanArgs a;
+    a.d = d; a.route = route; a.exist = exist; a.act_d = act_d; a.iteration = iteration; a.E = epochs; a.B = n_minibatches; a.M = M;
+    const int64_t per = (M + kMbMaxTiles - 1) / kMbMaxTiles;
+    a.tile = (per + kMbBlock - 1) / kMbBlock * kMbBlock;
+    a.tiles = (int)((M + a.tile - 1) / a.tile);
+    a.hist = (int32_t *)workspace; a.lists = lists; a.offsets = offsets; a.counts = counts;
+    cudaStream_t s = (cudaStream_t)stream;
+    k_mb_count<<<dim3((unsigned)a.tiles, (unsigned)epochs), kMbBlock, 0, s>>>(a);
+    api_count_launch();
+    int rc = ck(cudaGetLastError(), "k_mb_count");
+    if (rc) return rc;
+    k_mb_scan<<<dim3((unsigned)epochs, kMbRows), kMbMaxBuckets, 0, s>>>(a);
+    api_count_launch();
+    if ((rc = ck(cudaGetLastError(), "k_mb_scan"))) return rc;
+    k_mb_scatter<<<dim3((unsigned)a.tiles, (unsigned)epochs), kMbBlock, 0, s>>>(a);
+    api_count_launch();
+    return ck(cudaGetLastError(), "k_mb_scatter");
+}
+
 int mhppo_critic_grad_stats(int32_t n_in, const float *x, int32_t D, int64_t S, const int32_t *idx, int64_t K, int64_t CN,
                             const float *critic, const float *rtg, float inv_n, float *grad, double *loss, float *V, double *stats3,
                             void *workspace, void *stream) {

@@ -16,6 +16,7 @@
 // persistent CTA (one per SM).
 #pragma once
 #include "mlp.cuh"
+#include "ppo_rollout.cuh"      // policy_block: the minibatch plan draws from stream 3 of the policy-noise contract
 
 namespace mhppo {
 
@@ -565,6 +566,131 @@ __global__ void __launch_bounds__(192) k_reduce_gae(const double *__restrict__ p
     for (int b = lane; b < n; b += 32) acc += partial[(size_t)b * 6 + j];
     for (int o = 16; o > 0; o >>= 1) acc += __shfl_down_sync(0xffffffffu, acc, o);
     if (lane == 0) out[j] = acc;
+}
+
+// ---- minibatch plan (an option, Algo_PPO(n_minibatches=B); the reference's update is full-batch) --------------------------
+// In epoch e, column m = car*N + n (global env id g = env_id0 + n) goes to bucket
+//   b(car, g, e) = (w0 * B) >> 32,   w0 = word 0 of Philox4x32-10(counter = (e*C + car, 3 | iteration << 8, g_lo, g_hi), key = seed)
+// (stream 3 of the policy-noise contract, policy_block), so the buckets of an R-rank run are those of one rank holding all envs.
+// Per epoch the plan is a stable counting sort of the columns by bucket, for three selections at once (s = 0 cross: route 0,
+// 1 wait: route 1, 2 existing: exist != 0), plus the per-bucket counts of existing columns whose choice action is 0 / 1.
+// Within a bucket the columns are in ascending m.  Integer arithmetic in a fixed order throughout: the shared-memory histogram's
+// atomics add integers (order-free), and every list position comes from a scan or a warp ballot, never from an atomic.
+//   k_mb_count   grid (tiles, E): per-tile histogram [5][B] of one epoch -> hist[e][s][tile][b]
+//   k_mb_scan    grid (E, 5)    : per-bucket totals -> counts; exclusive scan over (b, tile) -> hist = each tile's base, offsets
+//   k_mb_scatter grid (tiles, E): rounds of 256 columns in m order, warp w after warp w-1, lanes ranked by __match_any_sync
+// Layouts: lists int32 [E][3][M], offsets int64 [E][3][B+1] (bucket b of selection s is lists[e][s][off[b] .. off[b+1])),
+// counts int64 [E][5][B] (rows: cross, wait, existing, existing with action 0, with action 1), workspace int32 [E][5][64][B].
+constexpr int kMbBlock = 256, kMbMaxTiles = 64, kMbMaxBuckets = 1024, kMbRows = 5;
+struct MbPlanArgs {
+    RolloutDims d;                       // N, C, env_id0 and the Philox key of the rollout
+    const int8_t *route, *exist;
+    const float *act_d;
+    uint32_t iteration;
+    int E, B, tiles;
+    int64_t M, tile;                     // columns, columns per tile (a multiple of kMbBlock)
+    int32_t *hist, *lists;
+    int64_t *offsets, *counts;
+};
+__device__ __forceinline__ int mb_bucket(const MbPlanArgs &a, int e, int64_t m, int &car) {
+    car = (int)(m / a.d.N);
+    const int64_t n = m - (int64_t)car * a.d.N;
+    const PhiloxBlock b = policy_block(a.d, n, (uint32_t)(e * a.d.C + car), 3u | (a.iteration << 8));
+    return (int)(((uint64_t)b.w0 * (uint64_t)a.B) >> 32);
+}
+// selection flags of column m: bit s set if the column belongs to selection s (0 cross, 1 wait, 2 existing, 3 / 4 action 0 / 1)
+__device__ __forceinline__ unsigned mb_flags(const MbPlanArgs &a, int64_t m) {
+    const int r = a.route[m];
+    const bool ex = a.exist[m] != 0;
+    const float ad = a.act_d[m];
+    return (r == 0 ? 1u : 0u) | (r == 1 ? 2u : 0u) | (ex ? 4u : 0u) | ((ex && ad == 0.f) ? 8u : 0u) | ((ex && ad == 1.f) ? 16u : 0u);
+}
+__global__ void __launch_bounds__(kMbBlock) k_mb_count(MbPlanArgs a) {
+    __shared__ int h[kMbRows * kMbMaxBuckets];
+    const int e = blockIdx.y, tile = blockIdx.x, B = a.B;
+    for (int i = threadIdx.x; i < kMbRows * B; i += kMbBlock) h[i] = 0;
+    __syncthreads();
+    const int64_t m0 = (int64_t)tile * a.tile, m1 = (m0 + a.tile < a.M) ? m0 + a.tile : a.M;
+    for (int64_t m = m0 + threadIdx.x; m < m1; m += kMbBlock) {
+        const unsigned f = mb_flags(a, m);
+        if (!f) continue;
+        int car;
+        const int b = mb_bucket(a, e, m, car);
+#pragma unroll
+        for (int s = 0; s < kMbRows; ++s)
+            if (f & (1u << s)) atomicAdd(&h[s * B + b], 1);
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < kMbRows * B; i += kMbBlock) {
+        const int s = i / B, b = i - s * B;
+        a.hist[(((size_t)e * kMbRows + s) * kMbMaxTiles + tile) * B + b] = h[i];
+    }
+}
+__global__ void __launch_bounds__(kMbMaxBuckets) k_mb_scan(MbPlanArgs a) {
+    __shared__ int64_t wsum[kMbMaxBuckets / 32];
+    const int e = blockIdx.x, s = blockIdx.y, B = a.B, b = threadIdx.x, lane = b & 31, w = b >> 5;
+    int32_t *h = a.hist + ((size_t)e * kMbRows + s) * kMbMaxTiles * B;
+    int64_t tot = 0;
+    if (b < B)
+        for (int t = 0; t < a.tiles; ++t) tot += h[(size_t)t * B + b];
+    if (b < B) a.counts[((size_t)e * kMbRows + s) * B + b] = tot;
+    if (s >= 3) return;                  // action counts: totals only
+    // exclusive scan of tot over b (warp shuffles, then the warp sums)
+    int64_t inc = tot;
+    for (int o = 1; o < 32; o <<= 1) { const int64_t v = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += v; }
+    if (lane == 31) wsum[w] = inc;
+    __syncthreads();
+    if (w == 0) {
+        int64_t x = wsum[lane], xi = x;
+        for (int o = 1; o < 32; o <<= 1) { const int64_t v = __shfl_up_sync(0xffffffffu, xi, o); if (lane >= o) xi += v; }
+        wsum[lane] = xi - x;             // exclusive prefix of the warp sums
+    }
+    __syncthreads();
+    if (b >= B) return;
+    int64_t base = wsum[w] + inc - tot;
+    int64_t *off = a.offsets + ((size_t)e * 3 + s) * (B + 1);
+    off[b] = base;
+    if (b == B - 1) off[B] = base + tot;
+    for (int t = 0; t < a.tiles; ++t) { const int v = h[(size_t)t * B + b]; h[(size_t)t * B + b] = (int32_t)base; base += v; }
+}
+__global__ void __launch_bounds__(kMbBlock) k_mb_scatter(MbPlanArgs a) {
+    __shared__ int run[3 * kMbMaxBuckets];
+    const int e = blockIdx.y, tile = blockIdx.x, B = a.B, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (int i = threadIdx.x; i < 3 * B; i += kMbBlock) {
+        const int s = i / B, b = i - s * B;
+        run[i] = a.hist[(((size_t)e * kMbRows + s) * kMbMaxTiles + tile) * B + b];
+    }
+    __syncthreads();
+    const int64_t m0 = (int64_t)tile * a.tile, m1 = (m0 + a.tile < a.M) ? m0 + a.tile : a.M;
+    const unsigned lt = (1u << lane) - 1u;
+    for (int64_t r0 = m0; r0 < m1; r0 += kMbBlock) {          // the same trip count in every thread of the CTA
+        const int64_t m = r0 + threadIdx.x;
+        const unsigned f = (m < m1) ? mb_flags(a, m) : 0u;
+        int car, b = 0;
+        if (f & 7u) b = mb_bucket(a, e, m, car);
+        int key[3], pos[3] = {0, 0, 0};
+        unsigned peers[3];
+#pragma unroll
+        for (int s = 0; s < 3; ++s) {
+            key[s] = (f & (1u << s)) ? b : -1;
+            peers[s] = __match_any_sync(0xffffffffu, key[s]);
+        }
+        for (int w = 0; w < kMbBlock / 32; ++w) {             // warps in m order: warp w takes its slots after warp w - 1
+            if (warp == w) {
+#pragma unroll
+                for (int s = 0; s < 3; ++s) {
+                    const int leader = __ffs(peers[s]) - 1;
+                    int base = 0;
+                    if (lane == leader && key[s] >= 0) { base = run[s * B + key[s]]; run[s * B + key[s]] = base + __popc(peers[s]); }
+                    pos[s] = __shfl_sync(0xffffffffu, base, leader) + __popc(peers[s] & lt);
+                }
+            }
+            __syncthreads();
+        }
+#pragma unroll
+        for (int s = 0; s < 3; ++s)
+            if (key[s] >= 0) a.lists[((size_t)e * 3 + s) * a.M + pos[s]] = (int32_t)m;
+    }
 }
 
 // ---- 6. Adam (torch.optim.Adam defaults, PY:719-724): p -= step_size * m / (sqrt(v) * inv_sqrt_bc2 + eps) ----

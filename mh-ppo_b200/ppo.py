@@ -7,6 +7,11 @@ Two options beyond the reference, both off by default (DESIGN.md §4 "GAE and en
   gae_lambda=None   a number in [0, 1]: the cross / wait nets train on GAE(gamma, lambda) returns and advantages, formed
                     once per update from the critics before the update (Env_rollout.gae); the choice net is unchanged
   entropy_coef=0.0  c > 0: the choice actor's loss gets the entropy bonus -c * mean_s H(pi(.|s))
+A third option, also off by default (DESIGN.md §4 "Minibatches"):
+  n_minibatches=None  an integer B in [1, 1024]: every epoch splits each net's columns ((car, env) trajectories) into B
+                    shuffled minibatches and takes one Adam step per minibatch instead of one full-batch step.  The buckets
+                    come from Philox stream 3 (mhppo_minibatch_plan), identical for any number of ranks; a minibatch with
+                    fewer than 2 samples over all ranks takes no step.  The unused `batch_size` of the reference stays unused.
 
 One iteration = one 80-step episode in every env of the vectorised env.  Multi-GPU: one process per GPU, envs
 sharded per rank; the only collectives are the all-reduce of the three advantage statistics and of the flat
@@ -28,6 +33,7 @@ from .rollout import Env_rollout
 
 
 _USE_DIST = True
+MAX_MINIBATCHES = 1024       # mhppo_minibatch_plan: 5 x B histogram bins per tile in shared memory
 
 
 def set_distributed(on):
@@ -95,6 +101,7 @@ class Algo_PPO:
         self._loss = torch.zeros(2, dtype=torch.float64, device=dev)
         self.last_losses = {}
         self._sel_cache = {}
+        self._mb = {}                                    # minibatch plan buffers (n_minibatches mode)
         # one contiguous gradient buffer per (actor, critic) pair: a single all-reduce per epoch carries both
         self._gbuf = {}
         for name, actor, critic in (("cross", self.actor_net_cross, self.critic_net_cross), ("wait", self.actor_net_wait, self.critic_net_wait),
@@ -123,6 +130,7 @@ class Algo_PPO:
         self.critic_lr, self.actor_lr, self.critic_d_lr, self.actor_d_lr = 1e-3, 3e-4, 1e-3, 3e-4
         self.num_states_c, self.num_states_d, self.num_actions, self.mean, self.std, self.dt = 13, None, 1, -1.0, 3.0, 0.3
         self.gae_lambda, self.entropy_coef = None, 0.0                     # options beyond the reference (module docstring)
+        self.n_minibatches = None
         for k, v in hyperparameters.items():
             setattr(self, k, v)
 
@@ -136,6 +144,9 @@ class Algo_PPO:
                 raise ValueError("GAE needs gamma in [0, 1], got %r" % (self.gamma,))
         if not (real(c) and math.isfinite(float(c)) and float(c) >= 0.0):
             raise ValueError("entropy_coef must be a finite number >= 0, got %r" % (c,))
+        B = self.n_minibatches
+        if B is not None and not (isinstance(B, numbers.Integral) and not isinstance(B, bool) and 1 <= int(B) <= MAX_MINIBATCHES):
+            raise ValueError("n_minibatches must be None or an integer in [1, %d], got %r" % (MAX_MINIBATCHES, B))
 
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.env.device).cuda_stream)
@@ -163,33 +174,39 @@ class Algo_PPO:
         return self._sel_cache[k]
 
     def train_model_c(self, actor, critic, opti_actor, opti_critic, want):
-        r, L, st = self.rollout, _lib.lib(), self._stream()
-        ws = self._ws.data_ptr()
+        r = self.rollout
         idx, K = self._selection(want)                                      # K == 0 still runs (zero partials): other ranks may have samples
         n = self._global_count(want, K * (r.S // r.M))             # sample slots: S = T * M, M = C * N columns
         if n < 1:
             return False                                     # PY:869/874: the net is skipped when its buffer is empty
+        self._epoch_c(actor, critic, opti_actor, opti_critic, want, idx.data_ptr(), K, n)
+        return True
+
+    def _epoch_c(self, actor, critic, opti_actor, opti_critic, want, idx, K, n):
+        """One gradient step of the pair on the K local columns of the int32 list at device address `idx`; n = the sample
+        count over all ranks (the whole buffer, or one minibatch of it)."""
+        r, L, st = self.rollout, _lib.lib(), self._stream()
+        ws = self._ws.data_ptr()
         if self.gae_lambda is not None:
             # GAE: fixed targets ret and advantages ret - V_old of this update; the critic pass must not overwrite V_old
             stats = self._gae_stats()
-            check(L.mhppo_ppo_grad(13, 0, r.obs_c.data_ptr(), 13, r.S, idx.data_ptr(), K, r.M, critic.flat.data_ptr(), None, None,
+            check(L.mhppo_ppo_grad(13, 0, r.obs_c.data_ptr(), 13, r.S, idx, K, r.M, critic.flat.data_ptr(), None, None,
                                    r.ret.data_ptr(), None, 0.0, 0.0, 1.0 / n, 0.0, 0.0, critic.grad.data_ptr(), self._loss.data_ptr() + 8,
                                    ws, st))
-            check(L.mhppo_ppo_grad_dev(13, 1, r.obs_c.data_ptr(), 13, r.S, idx.data_ptr(), K, r.M, actor.flat.data_ptr(),
+            check(L.mhppo_ppo_grad_dev(13, 1, r.obs_c.data_ptr(), 13, r.S, idx, K, r.M, actor.flat.data_ptr(),
                                        r.act.data_ptr(), r.logp.data_ptr(), r.ret.data_ptr(), r.V.data_ptr(), stats.data_ptr() + 24 * want,
                                        1.0 / n, 0.0, 0.0, actor.grad.data_ptr(), self._loss.data_ptr(), ws, st))
             self._step_pair(actor, critic, opti_actor, opti_critic)
-            return True
+            return
         # critic pass first: its forward is V = critic(s) of PY:785, so the same kernel returns V and the advantage statistics
-        check(L.mhppo_critic_grad_stats(13, r.obs_c.data_ptr(), 13, r.S, idx.data_ptr(), K, r.M, critic.flat.data_ptr(),
+        check(L.mhppo_critic_grad_stats(13, r.obs_c.data_ptr(), 13, r.S, idx, K, r.M, critic.flat.data_ptr(),
                                         r.rtg.data_ptr(), 1.0 / n, critic.grad.data_ptr(), self._loss.data_ptr() + 8,
                                         r.V.data_ptr(), self._stats.data_ptr(), ws, st))
         allreduce_sum_(self._stats)                          # (sum A, sum A^2, n) over all ranks; normalised inside the actor kernel
-        check(L.mhppo_ppo_grad_dev(13, 1, r.obs_c.data_ptr(), 13, r.S, idx.data_ptr(), K, r.M, actor.flat.data_ptr(),
+        check(L.mhppo_ppo_grad_dev(13, 1, r.obs_c.data_ptr(), 13, r.S, idx, K, r.M, actor.flat.data_ptr(),
                                    r.act.data_ptr(), r.logp.data_ptr(), r.rtg.data_ptr(), r.V.data_ptr(), self._stats.data_ptr(), 1.0 / n,
                                    0.0, 0.0, actor.grad.data_ptr(), self._loss.data_ptr(), ws, st))
         self._step_pair(actor, critic, opti_actor, opti_critic)
-        return True
 
     def _prepare_gae(self):
         """GAE mode, once per update before the epochs: V_old of both critics, the returns and the advantage statistics of
@@ -213,28 +230,33 @@ class Algo_PPO:
 
     # -- one epoch of train_model_d (PY:818-851) on the choice buffer -------------------------------------------
     def train_model_d(self, actor, critic, opti_actor, opti_critic):
-        r, L, st = self.rollout, _lib.lib(), self._stream()
-        ws, D = self._ws.data_ptr(), r.shape_env_d
         idx, K = self._selection(None)
         n = self._global_count(None, K)
         if n < 1:
             return False
-        check(L.mhppo_critic_grad_stats(D, r.obs_d.data_ptr(), D, r.M, idx.data_ptr(), K, r.M, critic.flat.data_ptr(),
+        self._epoch_d(actor, critic, opti_actor, opti_critic, idx.data_ptr(), K, n, lambda: self._action_fractions(n))
+        return True
+
+    def _epoch_d(self, actor, critic, opti_actor, opti_critic, idx, K, n, fractions):
+        """One gradient step of the choice pair on the K local columns at device address `idx`; n = the sample count over all
+        ranks, fractions() = (f0, f1) of those n samples."""
+        r, L, st = self.rollout, _lib.lib(), self._stream()
+        ws, D = self._ws.data_ptr(), r.shape_env_d
+        check(L.mhppo_critic_grad_stats(D, r.obs_d.data_ptr(), D, r.M, idx, K, r.M, critic.flat.data_ptr(),
                                         r.rew_d.data_ptr(), 1.0 / n, critic.grad.data_ptr(), self._loss.data_ptr() + 8,
                                         r.V_d.data_ptr(), self._stats.data_ptr(), ws, st))
         allreduce_sum_(self._stats)
-        f0, f1 = self._action_fractions(n)
+        f0, f1 = fractions()
         if self.entropy_coef:
-            check(L.mhppo_ppo_grad_ent(D, 2, r.obs_d.data_ptr(), D, r.M, idx.data_ptr(), K, r.M, actor.flat.data_ptr(),
+            check(L.mhppo_ppo_grad_ent(D, 2, r.obs_d.data_ptr(), D, r.M, idx, K, r.M, actor.flat.data_ptr(),
                                        r.act_d.data_ptr(), r.logp_d.data_ptr(), r.rew_d.data_ptr(), r.V_d.data_ptr(), self._stats.data_ptr(),
                                        1.0 / n, f0, f1, float(self.entropy_coef), actor.grad.data_ptr(), self._loss.data_ptr(), ws, st))
             self._step_pair(actor, critic, opti_actor, opti_critic)
-            return True
-        check(L.mhppo_ppo_grad_dev(D, 2, r.obs_d.data_ptr(), D, r.M, idx.data_ptr(), K, r.M, actor.flat.data_ptr(),
+            return
+        check(L.mhppo_ppo_grad_dev(D, 2, r.obs_d.data_ptr(), D, r.M, idx, K, r.M, actor.flat.data_ptr(),
                                    r.act_d.data_ptr(), r.logp_d.data_ptr(), r.rew_d.data_ptr(), r.V_d.data_ptr(), self._stats.data_ptr(),
                                    1.0 / n, f0, f1, actor.grad.data_ptr(), self._loss.data_ptr(), ws, st))
         self._step_pair(actor, critic, opti_actor, opti_critic)
-        return True
 
     def _action_fractions(self, n):
         """Fractions of the choice samples (all ranks) whose action is 0 / 1: the (M, M) broadcast of PY:834-842 collapses to
@@ -248,20 +270,71 @@ class Algo_PPO:
         return self._sel_cache["f01"]
 
     def update(self, epochs=10):
-        """The update half of train() (PY:866-882): 10 x (cross, wait) then 10 x choice."""
+        """The update half of train() (PY:866-882): 10 x (cross, wait) then 10 x choice; with n_minibatches = B, B steps per net
+        and epoch (_update_minibatches)."""
         self.rollout.value_std = self.value_std
         self.rollout._set_head(self.actor_net_cross)
         self.rollout.futur_rewards()                    # also the choice reward rew_d, which GAE mode uses too
         if self.gae_lambda is not None:
             self._prepare_gae()
-        for _ in range(epochs):
-            self.train_model_c(self.actor_net_cross, self.critic_net_cross, self.optimizer_actor_cross, self.optimizer_critic_cross, 0)
-            self.train_model_c(self.actor_net_wait, self.critic_net_wait, self.optimizer_actor_wait, self.optimizer_critic_wait, 1)
-        for _ in range(epochs):
-            self.train_model_d(self.actor_net_choice, self.critic_net_choice, self.optimizer_actor_choice, self.optimizer_critic_choice)
+        if self.n_minibatches is not None:
+            self._update_minibatches(epochs)
+        else:
+            for _ in range(epochs):
+                self.train_model_c(self.actor_net_cross, self.critic_net_cross, self.optimizer_actor_cross, self.optimizer_critic_cross, 0)
+                self.train_model_c(self.actor_net_wait, self.critic_net_wait, self.optimizer_actor_wait, self.optimizer_critic_wait, 1)
+            for _ in range(epochs):
+                self.train_model_d(self.actor_net_choice, self.critic_net_choice, self.optimizer_actor_choice, self.optimizer_critic_choice)
         if _lib.lib().mhppo_tc_failures():              # a tensor-core kernel gave up waiting for its MMAs: its gradients are garbage
             raise RuntimeError("a tcgen05 kernel of the update timed out on its mbarrier; the parameters of this update are not "
                                "trustworthy (reload a checkpoint; MHPPO_MLP=ffma selects the CUDA-core kernels)")
+
+    # -- minibatch mode (n_minibatches = B) ----------------------------------------------------------------------
+    def minibatch_plan(self, epochs):
+        """The plan of this update (mhppo_minibatch_plan on the last rollout): per epoch the bucket-major column lists of the
+        cross, wait and existing-car selections.  Returns (local, global) int64 numpy arrays [epochs][5][B] of the bucket sizes
+        (rows: cross, wait, existing, existing with choice action 0, with action 1), this rank's and all ranks' (one
+        all-reduce); the lists stay in self._mb["lists"] ([epochs][3][M] int32).  One device-to-host copy."""
+        r, B, dev = self.rollout, int(self.n_minibatches), self.rollout.route.device
+        if self._mb.get("key") != (epochs, B, r.M):
+            self._mb = dict(key=(epochs, B, r.M), lists=torch.empty(epochs * 3 * r.M, dtype=torch.int32, device=dev),
+                            offsets=torch.empty(epochs * 3 * (B + 1), dtype=torch.int64, device=dev),
+                            counts=torch.empty(2, epochs * 5 * B, dtype=torch.int64, device=dev),
+                            ws=torch.empty(1280 * epochs * B, dtype=torch.uint8, device=dev))
+        p = self._mb
+        check(_lib.lib().mhppo_minibatch_plan(C.byref(r._cfg), r.route.data_ptr(), r.exist.data_ptr(), r.act_d.data_ptr(),
+                                              (r.iteration - 1) & 0xFFFFFFFF, epochs, B, p["lists"].data_ptr(), p["offsets"].data_ptr(),
+                                              p["counts"].data_ptr(), p["ws"].data_ptr(), self._stream()))
+        p["counts"][1].copy_(p["counts"][0])
+        allreduce_sum_(p["counts"][1])
+        cnt = p["counts"].cpu().numpy().reshape(2, epochs, 5, B)
+        return cnt[0], cnt[1]
+
+    def _update_minibatches(self, epochs):
+        """Per epoch: cross on buckets 0..B-1, then wait on buckets 0..B-1; then the choice epochs on the existing cars.  Each
+        minibatch is one call of the epoch body on its slice of the plan's list, with n = its sample count over all ranks; one
+        with n < 2 takes no step (its unbiased std would be NaN).  Every rank takes the same decisions from the global counts."""
+        r, B = self.rollout, int(self.n_minibatches)
+        loc, glob = self.minibatch_plan(epochs)
+        base, T = self._mb["lists"].data_ptr(), r.S // r.M
+
+        def slices(e, s):
+            off = np.concatenate(([0], np.cumsum(loc[e, s])))
+            for b in range(B):
+                yield b, base + 4 * ((e * 3 + s) * r.M + int(off[b])), int(loc[e, s, b]), int(glob[e, s, b])
+        pairs = ((0, self.actor_net_cross, self.critic_net_cross, self.optimizer_actor_cross, self.optimizer_critic_cross),
+                 (1, self.actor_net_wait, self.critic_net_wait, self.optimizer_actor_wait, self.optimizer_critic_wait))
+        for e in range(epochs):
+            for want, actor, critic, oa, oc in pairs:
+                for b, idx, K, g in slices(e, want):
+                    if T * g >= 2:
+                        self._epoch_c(actor, critic, oa, oc, want, idx, K, T * g)
+        for e in range(epochs):
+            for b, idx, K, n in slices(e, 2):
+                if n >= 2:          # f0, f1 as _action_fractions forms them (float(count) / n): B = 1 is the default path bit for bit
+                    f01 = (float(glob[e, 3, b]) / n, float(glob[e, 4, b]) / n)
+                    self._epoch_d(self.actor_net_choice, self.critic_net_choice, self.optimizer_actor_choice, self.optimizer_critic_choice,
+                                  idx, K, n, lambda f01=f01: f01)
 
     # file-name stems of the three drivers: PY:908 / NB2 (coop) / NB1 (naif, "acc6")
     _STEM = {"coop_scalable": "pappo-scalable-coop", "coop": "pappo-coop", "naif": "pappo-acc6", "stop": "pappo-acc6"}
