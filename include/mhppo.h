@@ -292,6 +292,40 @@ int mhppo_adam2(float *p0_dev, const float *g0_dev, float *m0_dev, float *v0_dev
                 const float *g1_dev, float *m1_dev, float *v1_dev, int32_t n1, float lr1, int32_t step1, float beta1, float beta2,
                 float eps, void *stream);
 
+/* Update diagnostics (an option, Algo_PPO(diagnostics=True) / Algo_PPO(target_kl=delta); the reference logs nothing about its
+ * update).  The two passes below are mhppo_critic_grad_stats / mhppo_ppo_grad (head 0, GAE mode) and mhppo_ppo_grad_ent with the
+ * same gradient, loss and statistics outputs bit for bit; in the same kernel pass they also sum, per step (one Adam step of a pair),
+ * over this rank's samples, at the parameters before the step, and write into the step's RECORD ROW (fp64 [10], caller-zeroed):
+ *   [0] actor loss  [1] critic loss  (the values loss_dev receives)
+ *   [2] sum k3 = r - 1 - log r, log r = log pi(a_s|s) - logp_old[s] (Gaussian heads: the loss's log-prob; choice head: the
+ *       log-softmax of the TAKEN action act_dev[s]), fp32 log r, k3 in fp64 as expm1(log r) - log r
+ *   [3] count of r < 0.8 or r > 1.2 on the fp32 ratio the loss's clamp sees (choice: p_a * exp(-logp_old))
+ *   [4] sum H(pi(.|s)) (head 2 only, log-softmax form; 0 otherwise)
+ *   [5] sum (R - V)  [6] sum (R - V)^2  [7] sum R  [8] sum R^2   (R = rtg_dev, the critic's target; V = this pass's forward)
+ *   [9] taken: 1.0 once mhppo_adam2_halt takes the step (written by nothing else)
+ * Per-CTA fp64 partials, reduced in a fixed order by one more kernel per pass (no floating-point atomics): repeatable bit for
+ * bit.  Ratios (approx_kl = [2] / n, clip fraction = [3] / n, entropy = [4] / n, explained variance = 1 - Var(R-V) / Var(R)) are
+ * formed by the caller from the sums over all ranks.
+ * critic_grad_diag: V_dev and stats3_dev both given = mhppo_critic_grad_stats; both NULL = the critic pass of GAE mode, which does
+ * not write V. */
+int mhppo_critic_grad_diag(int32_t n_in, const float *x_dev, int32_t D, int64_t S, const int32_t *idx_dev, int64_t K, int64_t CN,
+                           const float *critic_dev, const float *rtg_dev, float inv_n, float *grad_dev, double *loss_dev,
+                           float *V_dev, double *stats3_dev, double *record_row_dev, void *workspace_dev, void *stream);
+/* ppo_grad_diag: the actor pass (head 1 or 2) of mhppo_ppo_grad_ent with the diagnostics above; kl_slot_dev (may be NULL) receives
+ * record[2] as fp32 -- place it behind the pair's packed gradients so that the gradient all-reduce also sums it over the ranks. */
+int mhppo_ppo_grad_diag(int32_t n_in, int32_t head, const float *x_dev, int32_t D, int64_t S, const int32_t *idx_dev, int64_t K,
+                        int64_t CN, const float *net_dev, const float *act_dev, const float *logp_old_dev, const float *rtg_dev,
+                        const float *V_dev, const double *adv_stats_dev, float inv_n, float f0, float f1, float ent_coef,
+                        float *grad_dev, double *loss_dev, float *kl_slot_dev, double *record_row_dev, void *workspace_dev,
+                        void *stream);
+/* mhppo_adam2 with the target-KL halt of SB3, checked before the step: if *halt_dev != 0 (int32, zeroed by the caller at the start of
+ * an update) nothing happens; else if *kl_sum_dev (the all-reduced fp32 k3 sum of the step) > kl_limit (= 1.5 * target_kl * n) the
+ * step is not taken and *halt_dev = 1, so every later launch with this flag does nothing; else both Adam steps are taken, with
+ * mhppo_adam2's arithmetic, and record_row_dev[9] = 1.0.  No host round trip. */
+int mhppo_adam2_halt(float *p0_dev, const float *g0_dev, float *m0_dev, float *v0_dev, int32_t n0, float lr0, int32_t step0, float *p1_dev,
+                     const float *g1_dev, float *m1_dev, float *v1_dev, int32_t n1, float lr1, int32_t step1, float beta1, float beta2,
+                     float eps, const float *kl_sum_dev, double kl_limit, int32_t *halt_dev, double *record_row_dev, void *stream);
+
 /* Self-test of the tcgen05 / TMEM building blocks behind the policy GEMMs: D[128,N] = A[128,K] * B[N,K]^T on one CTA,
  * mode 0 = one tf32 pass, mode 1 = 3xTF32 split accumulation.  (N,K) in {(64,32),(32,64),(64,16),(16,32)}. */
 /* implementation of the 13-input nets' kernels: 0 auto (tcgen05 for the update: forward + backward-data of ppo_grad /

@@ -78,7 +78,7 @@ static RolloutDims dims_of(const mhppo_rollout_cfg *c) {
     d.head = g_head;
     return d;
 }
-struct Workspace { float *gpartial; double *lpartial; double *spartial; };
+struct Workspace { float *gpartial; double *lpartial; double *spartial; double *dpartial; };
 static Workspace carve(void *ws, int KP) {
     Workspace w;
     w.gpartial = (float *)ws;
@@ -86,6 +86,7 @@ static Workspace carve(void *ws, int KP) {
     off = (off + 15) & ~(size_t)15;
     w.lpartial = (double *)((char *)ws + off);
     w.spartial = w.lpartial + kUpdateGridMax;
+    w.dpartial = w.spartial + (size_t)kUpdateGridMax * 3;      // [grid][kDiagW], the DIAG instances only
     return w;
 }
 }  // namespace mhppo
@@ -99,23 +100,24 @@ using namespace mhppo;
     } while (0)
 
 // 13-input nets, heads 0 / 1: forward and backward-data on the tensor cores (tc_grad.cuh) unless MHPPO_MLP=ffma
+template <bool DIAG>
 static int launch_grad_tc(int head, const SampleSet &ss, const float *net, const LossArgs &la, const Workspace &w, cudaStream_t s) {
     const size_t sm = sizeof(float) * kTcGradSmemFloats;
-    if (head == 0) { SET_SMEM((k_ppo_grad_tc<0>), sm); k_ppo_grad_tc<0><<<kGradGrid, kTcGradBlock, sm, s>>>(ss, net, la, w.gpartial, w.lpartial, fail_flag()); }
-    else { SET_SMEM((k_ppo_grad_tc<1>), sm); k_ppo_grad_tc<1><<<kGradGrid, kTcGradBlock, sm, s>>>(ss, net, la, w.gpartial, w.lpartial, fail_flag()); }
+    if (head == 0) { SET_SMEM((k_ppo_grad_tc<0, DIAG>), sm); k_ppo_grad_tc<0, DIAG><<<kGradGrid, kTcGradBlock, sm, s>>>(ss, net, la, w.gpartial, w.lpartial, fail_flag()); }
+    else { SET_SMEM((k_ppo_grad_tc<1, DIAG>), sm); k_ppo_grad_tc<1, DIAG><<<kGradGrid, kTcGradBlock, sm, s>>>(ss, net, la, w.gpartial, w.lpartial, fail_flag()); }
     api_count_launch();
     return ck(cudaGetLastError(), "k_ppo_grad_tc");
 }
 
-template <int KP>
+template <int KP, bool DIAG>
 static int launch_grad(int head, const SampleSet &ss, const float *net, const LossArgs &la, const Workspace &w, cudaStream_t s) {
     // (the tensor-core kernel stages exactly the 13 features of the cross / wait nets; a wider 16-padded input takes the FFMA kernel)
-    if (KP == 16 && ss.D <= 13 && head != 2 && use_tc(false)) return launch_grad_tc(head, ss, net, la, w, s);
+    if (KP == 16 && ss.D <= 13 && head != 2 && use_tc(false)) return launch_grad_tc<DIAG>(head, ss, net, la, w, s);
     const size_t sm = smem_grad<KP>();
-    if (head == 2 && la.ent_coef != 0.f) { SET_SMEM((k_ppo_grad<KP, 2, true>), sm); k_ppo_grad<KP, 2, true><<<kGradGrid, kMlpBlock, sm, s>>>(ss, net, la, w.gpartial, w.lpartial); }
-    else if (head == 0) { SET_SMEM((k_ppo_grad<KP, 0>), sm); k_ppo_grad<KP, 0><<<kGradGrid, kMlpBlock, sm, s>>>(ss, net, la, w.gpartial, w.lpartial); }
-    else if (head == 1) { SET_SMEM((k_ppo_grad<KP, 1>), sm); k_ppo_grad<KP, 1><<<kGradGrid, kMlpBlock, sm, s>>>(ss, net, la, w.gpartial, w.lpartial); }
-    else { SET_SMEM((k_ppo_grad<KP, 2>), sm); k_ppo_grad<KP, 2><<<kGradGrid, kMlpBlock, sm, s>>>(ss, net, la, w.gpartial, w.lpartial); }
+    if (head == 2 && la.ent_coef != 0.f) { SET_SMEM((k_ppo_grad<KP, 2, true, DIAG>), sm); k_ppo_grad<KP, 2, true, DIAG><<<kGradGrid, kMlpBlock, sm, s>>>(ss, net, la, w.gpartial, w.lpartial); }
+    else if (head == 0) { SET_SMEM((k_ppo_grad<KP, 0, false, DIAG>), sm); k_ppo_grad<KP, 0, false, DIAG><<<kGradGrid, kMlpBlock, sm, s>>>(ss, net, la, w.gpartial, w.lpartial); }
+    else if (head == 1) { SET_SMEM((k_ppo_grad<KP, 1, false, DIAG>), sm); k_ppo_grad<KP, 1, false, DIAG><<<kGradGrid, kMlpBlock, sm, s>>>(ss, net, la, w.gpartial, w.lpartial); }
+    else { SET_SMEM((k_ppo_grad<KP, 2, false, DIAG>), sm); k_ppo_grad<KP, 2, false, DIAG><<<kGradGrid, kMlpBlock, sm, s>>>(ss, net, la, w.gpartial, w.lpartial); }
     api_count_launch();
     return ck(cudaGetLastError(), "k_ppo_grad");
 }
@@ -319,7 +321,7 @@ int mhppo_tc_failures(void) {      /* 1 if any tensor-core kernel timed out wait
 int64_t mhppo_update_workspace_bytes(int32_t n_in) {
     const int kp = padded_in(n_in);
     if (kp < 0) return -1;
-    return (int64_t)(sizeof(float) * (size_t)kUpdateGridMax * net_params(kp) + 16 + sizeof(double) * (size_t)kUpdateGridMax * 4);
+    return (int64_t)(sizeof(float) * (size_t)kUpdateGridMax * net_params(kp) + 16 + sizeof(double) * (size_t)kUpdateGridMax * (4 + kDiagW));
 }
 
 static int make_set(SampleSet &ss, const float *x, int32_t D, int64_t S, const int32_t *idx, int64_t K, int64_t CN) {
@@ -353,7 +355,8 @@ int mhppo_value_stats(int32_t n_in, const float *x, int32_t D, int64_t S, const 
 static int ppo_grad_impl(int32_t n_in, int32_t head, const float *x, int32_t D, int64_t S, const int32_t *idx, int64_t K, int64_t CN,
                          const float *net, const float *act, const float *logp_old, const float *rtg, const float *V, float adv_mean,
                          float adv_inv_std, float inv_n, float f0, float f1, float *grad, double *loss, float *V_out, double *stats3,
-                         const double *adv_stats_dev, void *workspace, void *stream, float ent_coef = 0.f) {
+                         const double *adv_stats_dev, void *workspace, void *stream, float ent_coef = 0.f,
+                         double *diag_row = nullptr, float *kl_slot = nullptr) {
     if (!x || !net || !rtg || !grad || !loss || !workspace) return api_fail(MHPPO_EINVAL, "null argument");
     if (head < 0 || head > 2) return api_fail(MHPPO_EINVAL, "head must be 0, 1 or 2");
     if (head != 0 && (!act || !logp_old || !V)) return api_fail(MHPPO_EINVAL, "actor heads need act, logp_old and V");
@@ -364,14 +367,19 @@ static int ppo_grad_impl(int32_t n_in, int32_t head, const float *x, int32_t D, 
     const Workspace w = carve(workspace, kp);
     LossArgs la; la.act = act; la.logp_old = logp_old; la.rtg = rtg; la.V = V; la.adv_mean = adv_mean; la.adv_inv_std = adv_inv_std;
     la.inv_n = inv_n; la.f0 = f0; la.f1 = f1; la.V_out = V_out; la.spartial = stats3 ? w.spartial : nullptr;
-    la.head = g_head; la.stats_dev = adv_stats_dev; la.ent_coef = ent_coef;
+    la.head = g_head; la.stats_dev = adv_stats_dev; la.ent_coef = ent_coef; la.dpartial = w.dpartial;
     cudaStream_t s = (cudaStream_t)stream;
-    int rc = (kp == 16) ? launch_grad<16>(head, ss, net, la, w, s) : ((kp == 32) ? launch_grad<32>(head, ss, net, la, w, s) : launch_grad<56>(head, ss, net, la, w, s));
+    int rc;
+    if (diag_row) rc = (kp == 16) ? launch_grad<16, true>(head, ss, net, la, w, s) : ((kp == 32) ? launch_grad<32, true>(head, ss, net, la, w, s) : launch_grad<56, true>(head, ss, net, la, w, s));
+    else rc = (kp == 16) ? launch_grad<16, false>(head, ss, net, la, w, s) : ((kp == 32) ? launch_grad<32, false>(head, ss, net, la, w, s) : launch_grad<56, false>(head, ss, net, la, w, s));
     if (rc) return rc;
     const int npar = net_params(kp);
     k_reduce_all<<<(npar + 255) / 256, 256, 0, s>>>(w.gpartial, kGradGrid, npar, grad, w.lpartial, loss, w.spartial, stats3);
     api_count_launch();
-    return ck(cudaGetLastError(), "k_reduce_all");
+    if ((rc = ck(cudaGetLastError(), "k_reduce_all")) || !diag_row) return rc;
+    k_reduce_diag<<<1, 32, 0, s>>>(w.lpartial, w.dpartial, kGradGrid, head, diag_row, kl_slot);
+    api_count_launch();
+    return ck(cudaGetLastError(), "k_reduce_diag");
 }
 
 int mhppo_ppo_grad(int32_t n_in, int32_t head, const float *x, int32_t D, int64_t S, const int32_t *idx, int64_t K, int64_t CN,
@@ -399,6 +407,27 @@ int mhppo_ppo_grad_ent(int32_t n_in, int32_t head, const float *x, int32_t D, in
     if (ent_coef != 0.f && head != 2) return api_fail(MHPPO_EINVAL, "the entropy bonus needs head 2 (categorical choice actor)");
     return ppo_grad_impl(n_in, head, x, D, S, idx, K, CN, net, act, logp_old, rtg, V, 0.f, 0.f, inv_n, f0, f1, grad, loss, nullptr, nullptr,
                          adv_stats_dev, workspace, stream, ent_coef);
+}
+
+int mhppo_critic_grad_diag(int32_t n_in, const float *x, int32_t D, int64_t S, const int32_t *idx, int64_t K, int64_t CN,
+                           const float *critic, const float *rtg, float inv_n, float *grad, double *loss, float *V, double *stats3,
+                           double *record_row, void *workspace, void *stream) {
+    if (!record_row) return api_fail(MHPPO_EINVAL, "null argument");
+    if (!V != !stats3) return api_fail(MHPPO_EINVAL, "V and stats3 go together (both null: the critic pass of GAE mode)");
+    return ppo_grad_impl(n_in, 0, x, D, S, idx, K, CN, critic, nullptr, nullptr, rtg, nullptr, 0.f, 0.f, inv_n, 0.f, 0.f, grad, loss, V,
+                         stats3, nullptr, workspace, stream, 0.f, record_row, nullptr);
+}
+
+int mhppo_ppo_grad_diag(int32_t n_in, int32_t head, const float *x, int32_t D, int64_t S, const int32_t *idx, int64_t K, int64_t CN,
+                        const float *net, const float *act, const float *logp_old, const float *rtg, const float *V,
+                        const double *adv_stats_dev, float inv_n, float f0, float f1, float ent_coef, float *grad, double *loss,
+                        float *kl_slot, double *record_row, void *workspace, void *stream) {
+    if (!adv_stats_dev || !record_row) return api_fail(MHPPO_EINVAL, "null argument");
+    if (head != 1 && head != 2) return api_fail(MHPPO_EINVAL, "head must be 1 or 2 (the critic pass is mhppo_critic_grad_diag)");
+    if (!std::isfinite(ent_coef)) return api_fail(MHPPO_EINVAL, "ent_coef must be finite");
+    if (ent_coef != 0.f && head != 2) return api_fail(MHPPO_EINVAL, "the entropy bonus needs head 2 (categorical choice actor)");
+    return ppo_grad_impl(n_in, head, x, D, S, idx, K, CN, net, act, logp_old, rtg, V, 0.f, 0.f, inv_n, f0, f1, grad, loss, nullptr, nullptr,
+                         adv_stats_dev, workspace, stream, ent_coef, record_row, kl_slot);
 }
 
 int mhppo_gae(const float *rew, const float *V, const int8_t *route, int32_t T, int64_t CN, double gamma, double lambda, float *ret,
@@ -478,6 +507,24 @@ int mhppo_adam2(float *p0, const float *g0, float *m0, float *v0, int32_t n0, fl
     k_adam2<<<dim3((nmax + 255) / 256, 2), 256, 0, (cudaStream_t)stream>>>(mk(p0, g0, m0, v0, n0, lr0, step0), mk(p1, g1, m1, v1, n1, lr1, step1), beta1, beta2, eps);
     api_count_launch();
     return ck(cudaGetLastError(), "k_adam2");
+}
+
+int mhppo_adam2_halt(float *p0, const float *g0, float *m0, float *v0, int32_t n0, float lr0, int32_t step0, float *p1, const float *g1,
+                     float *m1, float *v1, int32_t n1, float lr1, int32_t step1, float beta1, float beta2, float eps,
+                     const float *kl_sum, double kl_limit, int32_t *halt, double *record_row, void *stream) {
+    if (!p0 || !g0 || !m0 || !v0 || !p1 || !g1 || !m1 || !v1 || n0 <= 0 || n1 <= 0 || step0 < 1 || step1 < 1) return api_fail(MHPPO_EINVAL, "bad argument");
+    if (!kl_sum || !halt || !record_row) return api_fail(MHPPO_EINVAL, "null argument");
+    if (std::isnan(kl_limit)) return api_fail(MHPPO_EINVAL, "kl_limit must not be NaN");
+    auto mk = [&](float *p, const float *g, float *m, float *v, int n, float lr, int step) {
+        const double bc1 = 1.0 - std::pow((double)beta1, (double)step), bc2 = 1.0 - std::pow((double)beta2, (double)step);
+        AdamArgs a; a.p = p; a.g = g; a.m = m; a.v = v; a.n = n; a.step_size = (float)((double)lr / bc1); a.inv_sqrt_bc2 = (float)(1.0 / std::sqrt(bc2));
+        return a;
+    };
+    const int nmax = n0 > n1 ? n0 : n1;
+    k_adam2_halt<<<dim3((nmax + 255) / 256, 2), 256, 0, (cudaStream_t)stream>>>(mk(p0, g0, m0, v0, n0, lr0, step0), mk(p1, g1, m1, v1, n1, lr1, step1),
+                                                                               beta1, beta2, eps, kl_sum, kl_limit, (int *)halt, record_row + 9);
+    api_count_launch();
+    return ck(cudaGetLastError(), "k_adam2_halt");
 }
 
 }  // extern "C"

@@ -96,6 +96,7 @@ struct LossArgs {
     const double *stats_dev;                   // actor heads, optional: (sum A, sum A^2, n) of the whole (all-rank) batch in device
                                                //   memory; adv_mean / adv_inv_std are then derived in the kernel (no host round trip)
     float ent_coef;                            // choice only: entropy bonus c; read only by the k_ppo_grad<KP, 2, true> instances
+    double *dpartial;                          // DIAG instances only: [grid][kDiagW] per-CTA diagnostic sums (LossAcc)
 };
 
 // advantage normalisation of PY:787 from the partial sums: mean, 1 / (unbiased std + 1e-10) (Algo_PPO.combine_stats)
@@ -236,18 +237,28 @@ __device__ __forceinline__ void wgrad_tile(float (&acc)[4][TJ], const float *__r
 // HEAD: 0 = critic (MSE), 1 = Gaussian actor (clipped surrogate), 2 = categorical actor with the (M,M) broadcast.
 // o: raw outputs of the net; returns dLoss/dz (4 padded outputs) and accumulates the loss and, for the critic,
 // the advantage statistics.
-struct LossAcc { double loss = 0.0, sA = 0.0, sAA = 0.0, cnt = 0.0; };
+// The DIAG instances also sum, per thread in fp64, the update diagnostics (DESIGN.md §4 "Diagnostics"): for the actor heads the
+// k3 estimator r - 1 - log r, the clipped-ratio count and (choice) the entropy; for the critic R - V, (R - V)^2, R and R^2.
+constexpr int kDiagW = 4;                  // diagnostic partials per CTA: actor (k3, clipped, H, 0), critic (R-V, (R-V)^2, R, R^2)
+struct LossAcc {
+    double loss = 0.0, sA = 0.0, sAA = 0.0, cnt = 0.0;
+    double d[kDiagW] = {0.0, 0.0, 0.0, 0.0};
+};
 // the per-sample inputs of the loss (rtg for every head; V, action, old log-prob for the actors): can be loaded ahead of use
 struct LossIn { float rtg, V, act, logp; };
-template <int HEAD>
+// (DIAG: the choice head also reads its taken action, for the per-sample ratio of the diagnostics)
+template <int HEAD, bool DIAG = false>
 __device__ __forceinline__ LossIn load_loss_in(const LossArgs &la, int64_t s) {
     LossIn in; in.rtg = la.rtg[s]; in.V = 0.f; in.act = 0.f; in.logp = 0.f;
     if (HEAD != 0) { in.V = la.V[s]; in.logp = la.logp_old[s]; }
-    if (HEAD == 1) in.act = la.act[s];
+    if (HEAD == 1 || (DIAG && HEAD == 2)) in.act = la.act[s];
     return in;
 }
-// ENT (HEAD == 2 only): adds the entropy bonus -c * inv_n * H(pi(.|s)) to the loss; ENT = false is the reference's loss
-template <int HEAD, bool ENT = false>
+// k3 = r - 1 - log r of an fp32 log-ratio, in fp64 as expm1(l) - l: no cancellation near r = 1, finite for |l| up to ~700
+__device__ __forceinline__ double k3_of(float l) { const double d = (double)l; return expm1(d) - d; }
+// ENT (HEAD == 2 only): adds the entropy bonus -c * inv_n * H(pi(.|s)) to the loss; ENT = false is the reference's loss.
+// DIAG: also accumulates the diagnostics of the sample into acc.d (read-only side computations: dz and acc.loss are unchanged)
+template <int HEAD, bool ENT = false, bool DIAG = false>
 __device__ __forceinline__ void ppo_loss(const LossArgs &la, int64_t s, const LossIn &in, float4 o, float (&dz)[OP], LossAcc &acc) {
     static_assert(!ENT || HEAD == 2, "the entropy bonus exists for the categorical head only");
     if (HEAD == 0) {                                           // critic_loss = MSE(V, rtg), PY:808-809
@@ -258,6 +269,10 @@ __device__ __forceinline__ void ppo_loss(const LossArgs &la, int64_t s, const Lo
             la.V_out[s] = o.x;
             const double A = (double)(in.rtg - o.x);
             acc.sA += A; acc.sAA += A * A; acc.cnt += 1.0;
+        }
+        if (DIAG) {                                            // explained variance: R = this pass's target, V = its forward output
+            const double R = (double)in.rtg, d = R - (double)o.x;
+            acc.d[0] += d; acc.d[1] += d * d; acc.d[2] += R; acc.d[3] += R * R;
         }
         return;
     }
@@ -270,6 +285,7 @@ __device__ __forceinline__ void ppo_loss(const LossArgs &la, int64_t s, const Lo
         const float s1 = ratio * An, s2 = fminf(fmaxf(ratio, 0.8f), 1.2f) * An;   // PY:804-805
         acc.loss += (double)(-fminf(s1, s2)) * (double)la.inv_n;                 // PY:806
         if (s1 <= s2) dz[0] = -la.inv_n * An * ratio * (2.0f * la.head.inv_2var * (a - mu)) * (la.head.std * (1.0f - th * th));
+        if (DIAG) { acc.d[0] += k3_of(lp - in.logp); acc.d[1] += (ratio < 0.8f || ratio > 1.2f) ? 1.0 : 0.0; }
     } else {
         // Categorical(probs [M,2]).log_prob(actions [M,1]) broadcasts to (M,M): lp[i,j] = log p_j(a_i)
         // (PY:834-842).  With two actions the mean over i collapses to the action frequencies f0, f1.
@@ -298,6 +314,25 @@ __device__ __forceinline__ void ppo_loss(const LossArgs &la, int64_t s, const Lo
             acc.loss -= (double)la.ent_coef * (double)la.inv_n * (double)H;
             dz[0] += ci * p0 * (lp0 + H); dz[1] += ci * p1 * (lp1 + H);
         }
+        if (DIAG) {
+            // the standard per-sample ratio of the taken action a_s (not the (M, M) broadcast the loss optimises): log r from the
+            // log-softmax, the clip test on the fp32 ratio p_a * exp(-logp_old) that the loss's clamp sees, H as in the ENT term
+            const float lse = logf(e0 + e1), lp0 = (o.x - m) - lse, lp1 = (o.y - m) - lse;
+            const bool a1 = in.act != 0.f;
+            const float rr = (a1 ? p1 : p0) * inv_old;
+            acc.d[0] += k3_of((a1 ? lp1 : lp0) - in.logp);
+            acc.d[1] += (rr < 0.8f || rr > 1.2f) ? 1.0 : 0.0;
+            acc.d[2] += (double)(-(p0 * lp0 + p1 * lp1));
+        }
+    }
+}
+
+// the CTA's diagnostic sums (team of nthreads) -> dpartial[blockIdx.x][0 .. kDiagW)
+__device__ __forceinline__ void write_diag_partials(const LossAcc &acc, double *__restrict__ dpartial, double *red, int tid, int nthreads) {
+#pragma unroll
+    for (int j = 0; j < kDiagW; ++j) {
+        const double t = team_sum(acc.d[j], red, tid, nthreads, 0);
+        if (tid == 0) dpartial[(size_t)blockIdx.x * kDiagW + j] = t;
     }
 }
 
@@ -376,7 +411,7 @@ struct WgradAcc {
     }
     // add the NG groups through `scratch` (>= net_params floats of shared memory no longer in use) and write the CTA's
     // partial gradient, loss and (critic) advantage statistics; `red` holds one double per warp of the CTA
-    template <int HEAD>
+    template <int HEAD, bool DIAG = false>
     __device__ __forceinline__ void finish(float *scratch, float *__restrict__ gpartial, double *__restrict__ lpartial, const LossArgs &la,
                                            const LossAcc &acc, double *red) const {
         constexpr int NPAR = net_params(KP), NT = 64 * NG;
@@ -394,13 +429,14 @@ struct WgradAcc {
             const double t0 = team_sum(acc.sA, red, tid, NT, 0), t1 = team_sum(acc.sAA, red, tid, NT, 0), t2 = team_sum(acc.cnt, red, tid, NT, 0);
             if (tid == 0) { la.spartial[blockIdx.x * 3 + 0] = t0; la.spartial[blockIdx.x * 3 + 1] = t1; la.spartial[blockIdx.x * 3 + 2] = t2; }
         }
+        if (DIAG) write_diag_partials(acc, la.dpartial, red, tid, NT);
     }
 };
 
 // Per tile: [thread = R samples] forward + loss + dz; then, layer by layer from the top, [register tiles] weight gradient from
 // (input activation, delta) and [thread = R samples] backward-data which overwrites the activation with its delta.
 constexpr int kTeams = 1;
-template <int KP, int HEAD, bool ENT = false>
+template <int KP, int HEAD, bool ENT = false, bool DIAG = false>
 __global__ void __launch_bounds__(kMlpBlock, 1) k_ppo_grad(SampleSet ss, const float *__restrict__ net, LossArgs la,
                                                            float *__restrict__ gpartial /* [grid][net_params] */,
                                                            double *__restrict__ lpartial /* [grid] */) {
@@ -456,7 +492,7 @@ __global__ void __launch_bounds__(kMlpBlock, 1) k_ppo_grad(SampleSet ss, const f
         for (int r = 0; r < R; ++r) {
             float *row = my + r * RS;
             float dz[OP] = {0.f, 0.f, 0.f, 0.f};
-            if (sel[r]) ppo_loss<HEAD, ENT>(la, sidx[r], load_loss_in<HEAD>(la, sidx[r]), ld4(row + G::D4), dz, acc);
+            if (sel[r]) ppo_loss<HEAD, ENT, DIAG>(la, sidx[r], load_loss_in<HEAD, DIAG>(la, sidx[r]), ld4(row + G::D4), dz, acc);
             // an unselected row has x = 0 but its activations are relu(bias) != 0: its dz = 0 keeps every gradient term zero
             st4(row + G::D4, make_float4(dz[0], dz[1], dz[2], dz[3]));
         }
@@ -476,7 +512,7 @@ __global__ void __launch_bounds__(kMlpBlock, 1) k_ppo_grad(SampleSet ss, const f
         wg.layer1_and_biases(rows, ROW, s0, HALF);
         __syncthreads();
     }
-    wg.template finish<HEAD>(rows, gpartial, lpartial, la, acc, red);
+    wg.template finish<HEAD, DIAG>(rows, gpartial, lpartial, la, acc, red);
 }
 
 // ---- 4. deterministic reduction of the per-CTA partials ----------------------------------------------
@@ -501,6 +537,23 @@ __global__ void __launch_bounds__(256) k_reduce_all(const float *__restrict__ gp
         const int j = threadIdx.x - 252;                                    // 0: loss, 1..3: sum A, sum A^2, n
         if (j == 0) { double acc = 0.0; for (int b = 0; b < nblocks; ++b) acc += lpartial[b]; *loss = acc; }
         else if (stats) { double acc = 0.0; for (int b = 0; b < nblocks; ++b) acc += spartial[(size_t)b * 3 + (j - 1)]; stats[j - 1] = acc; }
+    }
+}
+// the diagnostics of one ppo_grad launch with DIAG (after k_reduce_all, which it does not replace): fixed-order sums of the loss
+// and diagnostic partials into the step's fp64 record row (layout: include/mhppo.h, mhppo_ppo_grad_diag); the actor pass also
+// writes its k3 sum as fp32 to kl_slot (the slot behind the pair's packed gradients, all-reduced with them)
+__global__ void k_reduce_diag(const double *__restrict__ lpartial, const double *__restrict__ dpartial, int nblocks, int head,
+                              double *__restrict__ row, float *__restrict__ kl_slot) {
+    const int j = threadIdx.x;              // 0: loss, 1 .. kDiagW: the diagnostic columns
+    if (j > kDiagW) return;
+    double acc = 0.0;
+    if (j == 0) for (int b = 0; b < nblocks; ++b) acc += lpartial[b];
+    else for (int b = 0; b < nblocks; ++b) acc += dpartial[(size_t)b * kDiagW + (j - 1)];
+    if (head == 0) {
+        if (j == 0) row[1] = acc; else row[4 + j] = acc;           // critic loss; sum (R-V), (R-V)^2, R, R^2 -> row[5 .. 8]
+    } else {
+        if (j == 0) row[0] = acc; else if (j <= 3) row[1 + j] = acc;   // actor loss; sum k3, clipped, H -> row[2 .. 4]
+        if (j == 1 && kl_slot) *kl_slot = (float)acc;
     }
 }
 __global__ void k_reduce_scalars(const double *__restrict__ partial, int nblocks, int width, double *__restrict__ out) {
@@ -709,6 +762,26 @@ __global__ void __launch_bounds__(256) k_adam(float *__restrict__ p, const float
 // both Adam steps of one epoch (actor and critic of a pair act on different nets, PY:810-815) in one launch
 struct AdamArgs { float *p; const float *g; float *m, *v; int n; float step_size, inv_sqrt_bc2; };
 __global__ void __launch_bounds__(256) k_adam2(AdamArgs a0, AdamArgs a1, float beta1, float beta2, float eps) {
+    const AdamArgs a = blockIdx.y ? a1 : a0;
+    const int i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= a.n) return;
+    const float gi = a.g[i];
+    const float mi = beta1 * a.m[i] + (1.0f - beta1) * gi;
+    const float vi = beta2 * a.v[i] + (1.0f - beta2) * gi * gi;
+    a.m[i] = mi; a.v[i] = vi;
+    a.p[i] = a.p[i] - a.step_size * (mi / (sqrtf(vi) * a.inv_sqrt_bc2 + eps));
+}
+
+// both Adam steps of a pair with the target-KL halt (Algo_PPO(target_kl=delta)): *kl_sum = the pair's actor k3 sum over all
+// ranks (the fp32 slot behind its packed gradients); once it exceeds kl_limit = 1.5 delta n the pair is halted (*halt = 1) and
+// this and every later launch of the update leave p, m, v untouched.  Every block takes the same decision: a block that reads the
+// flag still 0 reads the same slot, and only a block that finds the limit exceeded writes the flag.  A step taken sets *taken = 1.
+// The element arithmetic is k_adam2's.
+__global__ void __launch_bounds__(256) k_adam2_halt(AdamArgs a0, AdamArgs a1, float beta1, float beta2, float eps,
+                                                    const float *__restrict__ kl_sum, double kl_limit, int *halt, double *taken) {
+    if (*(volatile int *)halt) return;
+    if ((double)*kl_sum > kl_limit) { if (threadIdx.x == 0) *(volatile int *)halt = 1; return; }
+    if (blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == 0) *taken = 1.0;
     const AdamArgs a = blockIdx.y ? a1 : a0;
     const int i = blockIdx.x * 256 + threadIdx.x;
     if (i >= a.n) return;

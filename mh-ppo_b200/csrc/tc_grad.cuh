@@ -87,7 +87,7 @@ __device__ __forceinline__ void bar_sync(int id, int n) { asm volatile("bar.sync
 // threads that leave the matching bar.sync, no extra fence needed)
 __device__ __forceinline__ void bar_arrive(int id, int n) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(n) : "memory"); }
 
-template <int HEAD>
+template <int HEAD, bool DIAG = false>
 __global__ void __launch_bounds__(kTcGradBlock, 1) k_ppo_grad_tc(SampleSet ss, const float *__restrict__ net, LossArgs la,
                                                               float *__restrict__ gpartial, double *__restrict__ lpartial,
                                                               int *__restrict__ fail_flag) {
@@ -287,7 +287,7 @@ __global__ void __launch_bounds__(kTcGradBlock, 1) k_ppo_grad_tc(SampleSet ss, c
                 }
                 // ---- loss epilogue -> dz (an unselected row keeps dz = 0: every gradient term of it vanishes)
                 float d4[OP] = {0.f, 0.f, 0.f, 0.f};
-                if (sel) ppo_loss<HEAD>(la, s, lcur, make_float4(o0, 0.f, 0.f, 0.f), d4, acc);
+                if (sel) ppo_loss<HEAD, false, DIAG>(la, s, lcur, make_float4(o0, 0.f, 0.f, 0.f), d4, acc);
                 st4(row + WG::D4, make_float4(d4[0], 0.f, 0.f, 0.f));
                 bar_arrive(BAR_R4, NT);                       // a3 and dz are in the rows: dW4 on W
 #pragma unroll
@@ -355,6 +355,7 @@ __global__ void __launch_bounds__(kTcGradBlock, 1) k_ppo_grad_tc(SampleSet ss, c
         const double t0 = team_sum(acc.sA, red, tid, NT, 0), t1 = team_sum(acc.sAA, red, tid, NT, 0), t2 = team_sum(acc.cnt, red, tid, NT, 0);
         if (tid == 0) { la.spartial[blockIdx.x * 3 + 0] = t0; la.spartial[blockIdx.x * 3 + 1] = t1; la.spartial[blockIdx.x * 3 + 2] = t2; }
     }
+    if (DIAG) write_diag_partials(acc, la.dpartial, red, tid, NT);
     tc::fence_before();
     __syncthreads();
     if ((threadIdx.x >> 5) == 0) tc::tmem_dealloc(tmem, 512);

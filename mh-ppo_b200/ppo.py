@@ -12,6 +12,12 @@ A third option, also off by default (DESIGN.md §4 "Minibatches"):
                     shuffled minibatches and takes one Adam step per minibatch instead of one full-batch step.  The buckets
                     come from Philox stream 3 (mhppo_minibatch_plan), identical for any number of ranks; a minibatch with
                     fewer than 2 samples over all ranks takes no step.  The unused `batch_size` of the reference stays unused.
+Two more, also off by default (DESIGN.md §4 "Diagnostics"):
+  diagnostics=False   True: every Adam step of an update gets a record (approx. KL, clip fraction, choice entropy, explained
+                      variance, both losses), computed on the device in the step's gradient pass; update() leaves them in
+                      `last_update_stats`, train() appends per-iteration means to `ep_diagnostics`.  No weight bit changes.
+  target_kl=None      delta > 0: a pair takes no further step in an update once a step's approx. KL exceeds 1.5 delta (SB3's
+                      rule, checked on the device before the step, no host round trip).  Turns the diagnostics on.
 
 One iteration = one 80-step episode in every env of the vectorised env.  Multi-GPU: one process per GPU, envs
 sharded per rank; the only collectives are the all-reduce of the three advantage statistics and of the flat
@@ -34,6 +40,22 @@ from .rollout import Env_rollout
 
 _USE_DIST = True
 MAX_MINIBATCHES = 1024       # mhppo_minibatch_plan: 5 x B histogram bins per tile in shared memory
+PAIRS = ("cross", "wait", "choice")
+DIAG_ROW = 10                # fp64 record row of one step (include/mhppo.h, mhppo_ppo_grad_diag)
+DIAG_FIELDS = [("epoch", np.int32), ("minibatch", np.int32), ("n", np.int64), ("actor_loss", np.float64), ("critic_loss", np.float64),
+               ("approx_kl", np.float64), ("clip_fraction", np.float64), ("entropy", np.float64), ("explained_variance", np.float64),
+               ("taken", np.bool_)]
+
+
+def diag_ratios(sums, n, choice):
+    """The diagnostics of one step from its record sums over all ranks (row layout of mhppo_ppo_grad_diag) and its sample count n:
+    approx_kl = mean k3, clip_fraction, entropy (choice pair only, NaN otherwise: the Gaussian heads have a fixed variance) and the
+    explained variance 1 - Var(R - V) / Var(R) with population variances, NaN when Var(R) = 0."""
+    sums = [float(v) for v in sums]
+    var_d = sums[6] / n - (sums[5] / n) ** 2
+    var_r = sums[8] / n - (sums[7] / n) ** 2
+    return dict(actor_loss=sums[0], critic_loss=sums[1], approx_kl=sums[2] / n, clip_fraction=sums[3] / n,
+                entropy=sums[4] / n if choice else float("nan"), explained_variance=1.0 - var_d / var_r if var_r > 0 else float("nan"))
 
 
 def set_distributed(on):
@@ -98,17 +120,24 @@ class Algo_PPO:
         nbytes = max(L.mhppo_update_workspace_bytes(self.num_states_c), L.mhppo_update_workspace_bytes(self.num_states_d))
         self._ws = torch.zeros(nbytes, dtype=torch.uint8, device=dev)
         self._stats = torch.zeros(3, dtype=torch.float64, device=dev)
+        self._diag = bool(self.diagnostics) or self.target_kl is not None
+        self._rec = None                                  # the record of the update in progress (diagnostics)
+        self._halt = torch.zeros(3, dtype=torch.int32, device=dev)
+        self.last_update_stats, self.ep_diagnostics = {}, []
         self._loss = torch.zeros(2, dtype=torch.float64, device=dev)
         self.last_losses = {}
         self._sel_cache = {}
         self._mb = {}                                    # minibatch plan buffers (n_minibatches mode)
-        # one contiguous gradient buffer per (actor, critic) pair: a single all-reduce per epoch carries both
-        self._gbuf = {}
+        # one contiguous gradient buffer per (actor, critic) pair: a single all-reduce per epoch carries both (with diagnostics also
+        # the actor's k3 sum in one more fp32 slot, which the target-KL halt reads)
+        self._gbuf, self._klslot = {}, {}
         for name, actor, critic in (("cross", self.actor_net_cross, self.critic_net_cross), ("wait", self.actor_net_wait, self.critic_net_wait),
                                     ("choice", self.actor_net_choice, self.critic_net_choice)):
-            g = torch.zeros(actor.n_param + critic.n_param, device=dev)
-            actor.grad, critic.grad = g[:actor.n_param], g[actor.n_param:]
+            np_ = actor.n_param + critic.n_param
+            g = torch.zeros(np_ + (1 if self._diag else 0), device=dev)
+            actor.grad, critic.grad = g[:actor.n_param], g[actor.n_param:np_]
             self._gbuf[id(actor)] = g
+            self._klslot[id(actor)] = g[np_:]
         self.sync_parameters()
 
     def sync_parameters(self):
@@ -131,6 +160,7 @@ class Algo_PPO:
         self.num_states_c, self.num_states_d, self.num_actions, self.mean, self.std, self.dt = 13, None, 1, -1.0, 3.0, 0.3
         self.gae_lambda, self.entropy_coef = None, 0.0                     # options beyond the reference (module docstring)
         self.n_minibatches = None
+        self.diagnostics, self.target_kl = False, None
         for k, v in hyperparameters.items():
             setattr(self, k, v)
 
@@ -147,6 +177,11 @@ class Algo_PPO:
         B = self.n_minibatches
         if B is not None and not (isinstance(B, numbers.Integral) and not isinstance(B, bool) and 1 <= int(B) <= MAX_MINIBATCHES):
             raise ValueError("n_minibatches must be None or an integer in [1, %d], got %r" % (MAX_MINIBATCHES, B))
+        if not isinstance(self.diagnostics, bool):
+            raise ValueError("diagnostics must be a bool, got %r" % (self.diagnostics,))
+        d = self.target_kl
+        if d is not None and not (real(d) and math.isfinite(float(d)) and float(d) > 0.0):
+            raise ValueError("target_kl must be None or a finite number > 0, got %r" % (d,))
 
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.env.device).cuda_stream)
@@ -187,26 +222,47 @@ class Algo_PPO:
         count over all ranks (the whole buffer, or one minibatch of it)."""
         r, L, st = self.rollout, _lib.lib(), self._stream()
         ws = self._ws.data_ptr()
+        row = self._diag_row(want, n)
         if self.gae_lambda is not None:
             # GAE: fixed targets ret and advantages ret - V_old of this update; the critic pass must not overwrite V_old
             stats = self._gae_stats()
-            check(L.mhppo_ppo_grad(13, 0, r.obs_c.data_ptr(), 13, r.S, idx, K, r.M, critic.flat.data_ptr(), None, None,
-                                   r.ret.data_ptr(), None, 0.0, 0.0, 1.0 / n, 0.0, 0.0, critic.grad.data_ptr(), self._loss.data_ptr() + 8,
-                                   ws, st))
-            check(L.mhppo_ppo_grad_dev(13, 1, r.obs_c.data_ptr(), 13, r.S, idx, K, r.M, actor.flat.data_ptr(),
-                                       r.act.data_ptr(), r.logp.data_ptr(), r.ret.data_ptr(), r.V.data_ptr(), stats.data_ptr() + 24 * want,
-                                       1.0 / n, 0.0, 0.0, actor.grad.data_ptr(), self._loss.data_ptr(), ws, st))
-            self._step_pair(actor, critic, opti_actor, opti_critic)
+            if row is not None:
+                check(L.mhppo_critic_grad_diag(13, r.obs_c.data_ptr(), 13, r.S, idx, K, r.M, critic.flat.data_ptr(), r.ret.data_ptr(), 1.0 / n,
+                                               critic.grad.data_ptr(), self._loss.data_ptr() + 8, None, None, row, ws, st))
+                self._actor_diag(1, r.obs_c, 13, r.S, idx, K, actor, r.act, r.logp, r.ret, r.V, stats.data_ptr() + 24 * want, n, 0.0, 0.0, 0.0, row)
+            else:
+                check(L.mhppo_ppo_grad(13, 0, r.obs_c.data_ptr(), 13, r.S, idx, K, r.M, critic.flat.data_ptr(), None, None,
+                                       r.ret.data_ptr(), None, 0.0, 0.0, 1.0 / n, 0.0, 0.0, critic.grad.data_ptr(), self._loss.data_ptr() + 8,
+                                       ws, st))
+                check(L.mhppo_ppo_grad_dev(13, 1, r.obs_c.data_ptr(), 13, r.S, idx, K, r.M, actor.flat.data_ptr(),
+                                           r.act.data_ptr(), r.logp.data_ptr(), r.ret.data_ptr(), r.V.data_ptr(), stats.data_ptr() + 24 * want,
+                                           1.0 / n, 0.0, 0.0, actor.grad.data_ptr(), self._loss.data_ptr(), ws, st))
+            self._step_pair(actor, critic, opti_actor, opti_critic, n, row)
             return
         # critic pass first: its forward is V = critic(s) of PY:785, so the same kernel returns V and the advantage statistics
-        check(L.mhppo_critic_grad_stats(13, r.obs_c.data_ptr(), 13, r.S, idx, K, r.M, critic.flat.data_ptr(),
-                                        r.rtg.data_ptr(), 1.0 / n, critic.grad.data_ptr(), self._loss.data_ptr() + 8,
-                                        r.V.data_ptr(), self._stats.data_ptr(), ws, st))
+        if row is not None:
+            check(L.mhppo_critic_grad_diag(13, r.obs_c.data_ptr(), 13, r.S, idx, K, r.M, critic.flat.data_ptr(), r.rtg.data_ptr(), 1.0 / n,
+                                           critic.grad.data_ptr(), self._loss.data_ptr() + 8, r.V.data_ptr(), self._stats.data_ptr(), row, ws, st))
+        else:
+            check(L.mhppo_critic_grad_stats(13, r.obs_c.data_ptr(), 13, r.S, idx, K, r.M, critic.flat.data_ptr(),
+                                            r.rtg.data_ptr(), 1.0 / n, critic.grad.data_ptr(), self._loss.data_ptr() + 8,
+                                            r.V.data_ptr(), self._stats.data_ptr(), ws, st))
         allreduce_sum_(self._stats)                          # (sum A, sum A^2, n) over all ranks; normalised inside the actor kernel
-        check(L.mhppo_ppo_grad_dev(13, 1, r.obs_c.data_ptr(), 13, r.S, idx, K, r.M, actor.flat.data_ptr(),
-                                   r.act.data_ptr(), r.logp.data_ptr(), r.rtg.data_ptr(), r.V.data_ptr(), self._stats.data_ptr(), 1.0 / n,
-                                   0.0, 0.0, actor.grad.data_ptr(), self._loss.data_ptr(), ws, st))
-        self._step_pair(actor, critic, opti_actor, opti_critic)
+        if row is not None:
+            self._actor_diag(1, r.obs_c, 13, r.S, idx, K, actor, r.act, r.logp, r.rtg, r.V, self._stats.data_ptr(), n, 0.0, 0.0, 0.0, row)
+        else:
+            check(L.mhppo_ppo_grad_dev(13, 1, r.obs_c.data_ptr(), 13, r.S, idx, K, r.M, actor.flat.data_ptr(),
+                                       r.act.data_ptr(), r.logp.data_ptr(), r.rtg.data_ptr(), r.V.data_ptr(), self._stats.data_ptr(), 1.0 / n,
+                                       0.0, 0.0, actor.grad.data_ptr(), self._loss.data_ptr(), ws, st))
+        self._step_pair(actor, critic, opti_actor, opti_critic, n, row)
+
+    def _actor_diag(self, head, x, D, S, idx, K, actor, act, logp, rtg, V, stats_ptr, n, f0, f1, c, row):
+        """The actor pass with diagnostics: record row `row` (device address) and the k3 sum into the pair's extra gradient slot."""
+        r = self.rollout
+        check(_lib.lib().mhppo_ppo_grad_diag(D, head, x.data_ptr(), D, S, idx, K, r.M, actor.flat.data_ptr(), act.data_ptr(), logp.data_ptr(),
+                                             rtg.data_ptr(), V.data_ptr(), stats_ptr, 1.0 / n, f0, f1, c, actor.grad.data_ptr(),
+                                             self._loss.data_ptr(), self._klslot[id(actor)].data_ptr(), row, self._ws.data_ptr(),
+                                             self._stream()))
 
     def _prepare_gae(self):
         """GAE mode, once per update before the epochs: V_old of both critics, the returns and the advantage statistics of
@@ -220,10 +276,19 @@ class Algo_PPO:
             self._prepare_gae()
         return self._sel_cache["gae"]
 
-    def _step_pair(self, actor, critic, opti_actor, opti_critic):
-        """All-reduce the pair's packed gradients (one collective) and take both Adam steps in one launch (PY:810-815)."""
+    def _step_pair(self, actor, critic, opti_actor, opti_critic, n=None, row=None):
+        """All-reduce the pair's packed gradients (one collective) and take both Adam steps in one launch (PY:810-815); with
+        target_kl, the launch that halts the pair on the device (its step counts are settled after the update, _diag_finish)."""
         allreduce_sum_(self._gbuf[id(actor)])
         actor.step += 1; critic.step += 1
+        if row is not None and self.target_kl is not None:
+            p = self._rec_pair
+            check(_lib.lib().mhppo_adam2_halt(actor.flat.data_ptr(), actor.grad.data_ptr(), actor.m.data_ptr(), actor.v.data_ptr(), actor.n_param,
+                                              opti_actor.lr, actor.step, critic.flat.data_ptr(), critic.grad.data_ptr(), critic.m.data_ptr(),
+                                              critic.v.data_ptr(), critic.n_param, opti_critic.lr, critic.step, 0.9, 0.999, 1e-8,
+                                              self._klslot[id(actor)].data_ptr(), 1.5 * float(self.target_kl) * n,
+                                              self._halt.data_ptr() + 4 * p, row, self._stream()))
+            return
         check(_lib.lib().mhppo_adam2(actor.flat.data_ptr(), actor.grad.data_ptr(), actor.m.data_ptr(), actor.v.data_ptr(), actor.n_param,
                                      opti_actor.lr, actor.step, critic.flat.data_ptr(), critic.grad.data_ptr(), critic.m.data_ptr(),
                                      critic.v.data_ptr(), critic.n_param, opti_critic.lr, critic.step, 0.9, 0.999, 1e-8, self._stream()))
@@ -242,11 +307,21 @@ class Algo_PPO:
         ranks, fractions() = (f0, f1) of those n samples."""
         r, L, st = self.rollout, _lib.lib(), self._stream()
         ws, D = self._ws.data_ptr(), r.shape_env_d
-        check(L.mhppo_critic_grad_stats(D, r.obs_d.data_ptr(), D, r.M, idx, K, r.M, critic.flat.data_ptr(),
-                                        r.rew_d.data_ptr(), 1.0 / n, critic.grad.data_ptr(), self._loss.data_ptr() + 8,
-                                        r.V_d.data_ptr(), self._stats.data_ptr(), ws, st))
+        row = self._diag_row(2, n)
+        if row is not None:
+            check(L.mhppo_critic_grad_diag(D, r.obs_d.data_ptr(), D, r.M, idx, K, r.M, critic.flat.data_ptr(), r.rew_d.data_ptr(), 1.0 / n,
+                                           critic.grad.data_ptr(), self._loss.data_ptr() + 8, r.V_d.data_ptr(), self._stats.data_ptr(), row, ws, st))
+        else:
+            check(L.mhppo_critic_grad_stats(D, r.obs_d.data_ptr(), D, r.M, idx, K, r.M, critic.flat.data_ptr(),
+                                            r.rew_d.data_ptr(), 1.0 / n, critic.grad.data_ptr(), self._loss.data_ptr() + 8,
+                                            r.V_d.data_ptr(), self._stats.data_ptr(), ws, st))
         allreduce_sum_(self._stats)
         f0, f1 = fractions()
+        if row is not None:
+            self._actor_diag(2, r.obs_d, D, r.M, idx, K, actor, r.act_d, r.logp_d, r.rew_d, r.V_d, self._stats.data_ptr(), n, f0, f1,
+                             float(self.entropy_coef), row)
+            self._step_pair(actor, critic, opti_actor, opti_critic, n, row)
+            return
         if self.entropy_coef:
             check(L.mhppo_ppo_grad_ent(D, 2, r.obs_d.data_ptr(), D, r.M, idx, K, r.M, actor.flat.data_ptr(),
                                        r.act_d.data_ptr(), r.logp_d.data_ptr(), r.rew_d.data_ptr(), r.V_d.data_ptr(), self._stats.data_ptr(),
@@ -277,17 +352,98 @@ class Algo_PPO:
         self.rollout.futur_rewards()                    # also the choice reward rew_d, which GAE mode uses too
         if self.gae_lambda is not None:
             self._prepare_gae()
-        if self.n_minibatches is not None:
-            self._update_minibatches(epochs)
-        else:
-            for _ in range(epochs):
-                self.train_model_c(self.actor_net_cross, self.critic_net_cross, self.optimizer_actor_cross, self.optimizer_critic_cross, 0)
-                self.train_model_c(self.actor_net_wait, self.critic_net_wait, self.optimizer_actor_wait, self.optimizer_critic_wait, 1)
-            for _ in range(epochs):
-                self.train_model_d(self.actor_net_choice, self.critic_net_choice, self.optimizer_actor_choice, self.optimizer_critic_choice)
-        if _lib.lib().mhppo_tc_failures():              # a tensor-core kernel gave up waiting for its MMAs: its gradients are garbage
+        if self._diag:
+            self._diag_begin(epochs)
+        try:
+            if self.n_minibatches is not None:
+                self._update_minibatches(epochs)
+            else:
+                for e in range(epochs):
+                    self._pos = (e, 0)
+                    self.train_model_c(self.actor_net_cross, self.critic_net_cross, self.optimizer_actor_cross, self.optimizer_critic_cross, 0)
+                    self.train_model_c(self.actor_net_wait, self.critic_net_wait, self.optimizer_actor_wait, self.optimizer_critic_wait, 1)
+                for e in range(epochs):
+                    self._pos = (e, 0)
+                    self.train_model_d(self.actor_net_choice, self.critic_net_choice, self.optimizer_actor_choice, self.optimizer_critic_choice)
+            pending = self._diag_fetch() if self._diag else None
+        finally:
+            self._rec = None                             # train_model_c / _d outside update() take the plain path
+        failed = _lib.lib().mhppo_tc_failures()          # (synchronises the device: the record's copy has landed with it)
+        if pending is not None:
+            host, done = pending
+            done.synchronize()
+            self._diag_finish(host.numpy())              # step counts settled even when the update is reported broken below
+        if failed:                                       # a tensor-core kernel gave up waiting for its MMAs: its gradients are garbage
             raise RuntimeError("a tcgen05 kernel of the update timed out on its mbarrier; the parameters of this update are not "
                                "trustworthy (reload a checkpoint; MHPPO_MLP=ffma selects the CUDA-core kernels)")
+
+    # -- diagnostics (diagnostics=True / target_kl) ---------------------------------------------------------------------
+    def _diag_begin(self, epochs):
+        """A zeroed record of one fp64 row per possible step of this update, the pairs' halt flags cleared."""
+        B = int(self.n_minibatches) if self.n_minibatches is not None else 1
+        self._rec = torch.zeros(3 * epochs * B, DIAG_ROW, dtype=torch.float64, device=self._stats.device)
+        self._rec_steps = {p: [] for p in PAIRS}        # per pair: (epoch, minibatch, n, record row), in launch order
+        self._rec_used = 0
+        self._rec_steps0 = {p: (a.step, c.step) for p, a, c in self._pair_nets()}
+        self._pos = (0, 0)
+        if self.target_kl is not None:
+            self._halt.zero_()
+
+    def _pair_nets(self):
+        return (("cross", self.actor_net_cross, self.critic_net_cross), ("wait", self.actor_net_wait, self.critic_net_wait),
+                ("choice", self.actor_net_choice, self.critic_net_choice))
+
+    def _diag_row(self, pair, n):
+        """Device address of the next record row for a step of pair 0 / 1 / 2 with n samples over all ranks; None outside update()
+        or without diagnostics."""
+        if self._rec is None:
+            return None
+        i = self._rec_used
+        self._rec_used += 1
+        self._rec_steps[PAIRS[pair]].append((self._pos[0], self._pos[1], int(n), i))
+        self._rec_pair = pair
+        return self._rec.data_ptr() + 8 * DIAG_ROW * i
+
+    def _diag_fetch(self):
+        """One all-reduce of the record's sums over the ranks (the taken flags are the same on every rank) and one asynchronous
+        device-to-host copy of the used rows into pinned memory; returns (host tensor, event of the copy).  The host waits for it
+        in the same synchronisation as the mhppo_tc_failures copy that ends every update."""
+        used = self._rec_used
+        if _dist() is not None and used:
+            s = self._rec[:used, :DIAG_ROW - 1].contiguous()
+            allreduce_sum_(s)
+            self._rec[:used, :DIAG_ROW - 1] = s
+        host = torch.empty((used, DIAG_ROW), dtype=torch.float64, pin_memory=True)
+        host.copy_(self._rec[:used], non_blocking=True)
+        done = torch.cuda.Event()
+        done.record(torch.cuda.current_stream(self._rec.device))
+        return host, done
+
+    def _diag_finish(self, host):
+        """last_update_stats from the copied record; with target_kl, each pair's Adam step counts become the steps it took."""
+        out = {}
+        for p, actor, critic in self._pair_nets():
+            steps = self._rec_steps[p]
+            a = np.zeros(len(steps), dtype=DIAG_FIELDS)
+            for j, (e, b, n, i) in enumerate(steps):
+                a[j]["epoch"], a[j]["minibatch"], a[j]["n"] = e, b, n
+                for k, v in diag_ratios(host[i, :DIAG_ROW - 1], n, p == "choice").items():
+                    a[j][k] = v
+                a[j]["taken"] = bool(host[i, DIAG_ROW - 1]) if self.target_kl is not None else True
+            out[p] = a
+            if self.target_kl is not None:
+                s0a, s0c = self._rec_steps0[p]
+                actor.step, critic.step = s0a + int(a["taken"].sum()), s0c + int(a["taken"].sum())
+        self.last_update_stats = out
+
+    def diagnostics_summary(self):
+        """Per pair: the means of last_update_stats' float fields over the launched steps, and the steps launched / taken."""
+        out = {}
+        for p, a in self.last_update_stats.items():
+            d = {k: (float(np.mean(a[k])) if len(a) else float("nan")) for k, t in DIAG_FIELDS if t is np.float64}
+            d["steps_launched"], d["steps_taken"] = int(len(a)), int(a["taken"].sum())
+            out[p] = d
+        return out
 
     # -- minibatch mode (n_minibatches = B) ----------------------------------------------------------------------
     def minibatch_plan(self, epochs):
@@ -327,10 +483,12 @@ class Algo_PPO:
         for e in range(epochs):
             for want, actor, critic, oa, oc in pairs:
                 for b, idx, K, g in slices(e, want):
+                    self._pos = (e, b)
                     if T * g >= 2:
                         self._epoch_c(actor, critic, oa, oc, want, idx, K, T * g)
         for e in range(epochs):
             for b, idx, K, n in slices(e, 2):
+                self._pos = (e, b)
                 if n >= 2:          # f0, f1 as _action_fractions forms them (float(count) / n): B = 1 is the default path bit for bit
                     f01 = (float(glob[e, 3, b]) / n, float(glob[e, 4, b]) / n)
                     self._epoch_d(self.actor_net_choice, self.critic_net_choice, self.optimizer_actor_choice, self.optimizer_critic_choice,
@@ -353,6 +511,8 @@ class Algo_PPO:
                 self.ep_reward_wait.append(float(wait))
             self.ep_reward_choice.append(float(choice))
             self.ep_scenario_balance.append([nc, nw])
+            if self._diag:
+                self.ep_diagnostics.append(self.diagnostics_summary())
             self.total_loop += 1
             if verbose:
                 print("Episode * {} * cross {:.4f} wait {:.4f} choice {:.4f}  (#cross {} #wait {})".format(
