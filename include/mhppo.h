@@ -302,7 +302,7 @@ int mhppo_adam2(float *p0_dev, const float *g0_dev, float *m0_dev, float *v0_dev
  *   [3] count of r < 0.8 or r > 1.2 on the fp32 ratio the loss's clamp sees (choice: p_a * exp(-logp_old))
  *   [4] sum H(pi(.|s)) (head 2 only, log-softmax form; 0 otherwise)
  *   [5] sum (R - V)  [6] sum (R - V)^2  [7] sum R  [8] sum R^2   (R = rtg_dev, the critic's target; V = this pass's forward)
- *   [9] taken: 1.0 once mhppo_adam2_halt takes the step (written by nothing else)
+ *   [9] taken: 1.0 once mhppo_adam2_halt (or mhppo_adam2_clip with the halt) takes the step (written by nothing else)
  * Per-CTA fp64 partials, reduced in a fixed order by one more kernel per pass (no floating-point atomics): repeatable bit for
  * bit.  Ratios (approx_kl = [2] / n, clip fraction = [3] / n, entropy = [4] / n, explained variance = 1 - Var(R-V) / Var(R)) are
  * formed by the caller from the sums over all ranks.
@@ -325,6 +325,21 @@ int mhppo_ppo_grad_diag(int32_t n_in, int32_t head, const float *x_dev, int32_t 
 int mhppo_adam2_halt(float *p0_dev, const float *g0_dev, float *m0_dev, float *v0_dev, int32_t n0, float lr0, int32_t step0, float *p1_dev,
                      const float *g1_dev, float *m1_dev, float *v1_dev, int32_t n1, float lr1, int32_t step1, float beta1, float beta2,
                      float eps, const float *kl_sum_dev, double kl_limit, int32_t *halt_dev, double *record_row_dev, void *stream);
+
+/* mhppo_adam2 with per-network gradient-norm clipping (an option, Algo_PPO(max_grad_norm=g); the reference does not clip), torch's
+ * clip_grad_norm_(net.parameters(), max_norm) before each net's step: norm = the fp64 L2 norm of the net's whole flat gradient
+ * (n0 / n1 floats; the padded slots of the flat layout are exactly 0 after every gradient pass, so it is the norm over the
+ * reference-layout tensors), coef = max_norm / (norm + 1e-6), and the Adam step uses coef * grad when coef < 1, else the gradient
+ * unchanged.  A non-finite norm gives coef = 1.  An unclipped step is mhppo_adam2's (mhppo_adam2_halt's) bit for bit; g0_dev and
+ * g1_dev are not written.  norms_out_dev (may be NULL): fp64 [2], actor (net 0) then critic (net 1).  kl_sum_dev, kl_limit, halt_dev,
+ * record_row_dev: mhppo_adam2_halt's halt, tested after the norms are written (a halted step still reports its norms); all three
+ * pointers NULL = no halt, kl_limit unused.  Sum of squares in a fixed order (no atomics): repeatable bit for bit.  One launch.
+ * MHPPO_EINVAL: mhppo_adam2's checks, max_norm NaN or <= 0 (+inf records the norms and never clips), some but not all halt
+ * pointers, kl_limit NaN with the halt. */
+int mhppo_adam2_clip(float *p0_dev, const float *g0_dev, float *m0_dev, float *v0_dev, int32_t n0, float lr0, int32_t step0, float *p1_dev,
+                     const float *g1_dev, float *m1_dev, float *v1_dev, int32_t n1, float lr1, int32_t step1, float beta1, float beta2,
+                     float eps, double max_norm, double *norms_out_dev, const float *kl_sum_dev, double kl_limit, int32_t *halt_dev,
+                     double *record_row_dev, void *stream);
 
 /* Self-test of the tcgen05 / TMEM building blocks behind the policy GEMMs: D[128,N] = A[128,K] * B[N,K]^T on one CTA,
  * mode 0 = one tf32 pass, mode 1 = 3xTF32 split accumulation.  (N,K) in {(64,32),(32,64),(64,16),(16,32)}. */

@@ -792,4 +792,50 @@ __global__ void __launch_bounds__(256) k_adam2_halt(AdamArgs a0, AdamArgs a1, fl
     a.p[i] = a.p[i] - a.step_size * (mi / (sqrtf(vi) * a.inv_sqrt_bc2 + eps));
 }
 
+// both Adam steps of a pair with per-network gradient-norm clipping (Algo_PPO(max_grad_norm=g)), torch's clip_grad_norm_ on each
+// net: norm = ||g||_2 over the net's whole flat gradient, coef = max_norm / (norm + 1e-6), and the step uses coef * g when coef < 1.
+// A non-finite norm (or max_norm = inf) gives coef = 1, the unclipped step.  One CTA per net (blockIdx.y), since the norm must be
+// known before any element steps: pass 1 sums g^2 in fp64 (each thread a fixed strided subset, then a shuffle tree per warp and
+// warp 0 over the warp sums: a fixed order, repeatable bit for bit), pass 2 is k_adam2's element arithmetic on g * coef (exact
+// for coef = 1, so an unclipped step is k_adam2's bit for bit).  g is not written.  norms_out[y] = norm when norms_out != NULL.
+// HALT: k_adam2_halt's halt on top, tested after the norms are written, so a step the halt skips still reports its norm.
+constexpr int kClipBlock = 1024;
+template <bool HALT>
+__global__ void __launch_bounds__(kClipBlock) k_adam2_clip(AdamArgs a0, AdamArgs a1, float beta1, float beta2, float eps, double max_norm,
+                                                           double *__restrict__ norms_out, const float *__restrict__ kl_sum,
+                                                           double kl_limit, int *halt, double *taken) {
+    __shared__ double wsum[kClipBlock / 32];
+    __shared__ float coef_s;
+    const AdamArgs a = blockIdx.y ? a1 : a0;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    double ss = 0.0;
+    for (int i = threadIdx.x; i < a.n; i += kClipBlock) { const double gi = (double)a.g[i]; ss += gi * gi; }
+    for (int o = 16; o > 0; o >>= 1) ss += __shfl_down_sync(0xffffffffu, ss, o);
+    if (lane == 0) wsum[warp] = ss;
+    __syncthreads();
+    if (warp == 0) {
+        double t = wsum[lane];
+        for (int o = 16; o > 0; o >>= 1) t += __shfl_down_sync(0xffffffffu, t, o);
+        if (lane == 0) {
+            const double norm = sqrt(t), c = max_norm / (norm + 1e-6);
+            coef_s = (isfinite(norm) && c < 1.0) ? (float)c : 1.0f;
+            if (norms_out) norms_out[blockIdx.y] = norm;
+        }
+    }
+    __syncthreads();
+    if (HALT) {
+        if (*(volatile int *)halt) return;
+        if ((double)*kl_sum > kl_limit) { if (threadIdx.x == 0) *(volatile int *)halt = 1; return; }
+        if (blockIdx.y == 0 && threadIdx.x == 0) *taken = 1.0;
+    }
+    const float coef = coef_s;
+    for (int i = threadIdx.x; i < a.n; i += kClipBlock) {
+        const float gi = a.g[i] * coef;
+        const float mi = beta1 * a.m[i] + (1.0f - beta1) * gi;
+        const float vi = beta2 * a.v[i] + (1.0f - beta2) * gi * gi;
+        a.m[i] = mi; a.v[i] = vi;
+        a.p[i] = a.p[i] - a.step_size * (mi / (sqrtf(vi) * a.inv_sqrt_bc2 + eps));
+    }
+}
+
 }  // namespace mhppo

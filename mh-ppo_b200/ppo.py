@@ -18,6 +18,13 @@ Two more, also off by default (DESIGN.md §4 "Diagnostics"):
                       `last_update_stats`, train() appends per-iteration means to `ep_diagnostics`.  No weight bit changes.
   target_kl=None      delta > 0: a pair takes no further step in an update once a step's approx. KL exceeds 1.5 delta (SB3's
                       rule, checked on the device before the step, no host round trip).  Turns the diagnostics on.
+One more, also off by default (DESIGN.md §5 "Gradient-norm clipping"):
+  max_grad_norm=None  g > 0 (+inf allowed): before each Adam step, each of the six nets' gradients is clipped on its own, as
+                      torch.nn.utils.clip_grad_norm_(net.parameters(), g) would before that net's optimiser step: with norm = the L2
+                      norm of the net's whole all-reduced gradient, the step uses g / (norm + 1e-6) * grad when that factor is < 1.
+                      A non-finite norm leaves the step unclipped; g = inf never clips.  Fused into the pair's Adam launch
+                      (mhppo_adam2_clip).  update() leaves every step's two norms in `last_grad_norms`, train() appends
+                      per-iteration means to `ep_grad_norms`.
 
 One iteration = one 80-step episode in every env of the vectorised env.  Multi-GPU: one process per GPU, envs
 sharded per rank; the only collectives are the all-reduce of the three advantage statistics and of the flat
@@ -45,6 +52,7 @@ DIAG_ROW = 10                # fp64 record row of one step (include/mhppo.h, mhp
 DIAG_FIELDS = [("epoch", np.int32), ("minibatch", np.int32), ("n", np.int64), ("actor_loss", np.float64), ("critic_loss", np.float64),
                ("approx_kl", np.float64), ("clip_fraction", np.float64), ("entropy", np.float64), ("explained_variance", np.float64),
                ("taken", np.bool_)]
+GRAD_NORM_FIELDS = [("epoch", np.int32), ("minibatch", np.int32), ("actor_grad_norm", np.float64), ("critic_grad_norm", np.float64)]
 
 
 def diag_ratios(sums, n, choice):
@@ -56,6 +64,15 @@ def diag_ratios(sums, n, choice):
     var_r = sums[8] / n - (sums[7] / n) ** 2
     return dict(actor_loss=sums[0], critic_loss=sums[1], approx_kl=sums[2] / n, clip_fraction=sums[3] / n,
                 entropy=sums[4] / n if choice else float("nan"), explained_variance=1.0 - var_d / var_r if var_r > 0 else float("nan"))
+
+
+def _to_host_async(t):
+    """An asynchronous device-to-host copy of t into pinned memory; returns (host tensor, event of the copy)."""
+    host = torch.empty(t.shape, dtype=t.dtype, pin_memory=True)
+    host.copy_(t, non_blocking=True)
+    done = torch.cuda.Event()
+    done.record(torch.cuda.current_stream(t.device))
+    return host, done
 
 
 def set_distributed(on):
@@ -121,9 +138,12 @@ class Algo_PPO:
         self._ws = torch.zeros(nbytes, dtype=torch.uint8, device=dev)
         self._stats = torch.zeros(3, dtype=torch.float64, device=dev)
         self._diag = bool(self.diagnostics) or self.target_kl is not None
+        self._steps = None                                # per pair, the steps of the update in progress (diagnostics, clipping)
         self._rec = None                                  # the record of the update in progress (diagnostics)
+        self._norms = None                                # its gradient norms, fp64 [step][actor, critic] (clipping)
         self._halt = torch.zeros(3, dtype=torch.int32, device=dev)
         self.last_update_stats, self.ep_diagnostics = {}, []
+        self.last_grad_norms, self.ep_grad_norms = {}, []
         self._loss = torch.zeros(2, dtype=torch.float64, device=dev)
         self.last_losses = {}
         self._sel_cache = {}
@@ -161,6 +181,7 @@ class Algo_PPO:
         self.gae_lambda, self.entropy_coef = None, 0.0                     # options beyond the reference (module docstring)
         self.n_minibatches = None
         self.diagnostics, self.target_kl = False, None
+        self.max_grad_norm = None
         for k, v in hyperparameters.items():
             setattr(self, k, v)
 
@@ -182,6 +203,9 @@ class Algo_PPO:
         d = self.target_kl
         if d is not None and not (real(d) and math.isfinite(float(d)) and float(d) > 0.0):
             raise ValueError("target_kl must be None or a finite number > 0, got %r" % (d,))
+        g = self.max_grad_norm
+        if g is not None and not (real(g) and float(g) > 0.0):
+            raise ValueError("max_grad_norm must be None or a number > 0 (inf: record the norms, never clip), got %r" % (g,))
 
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.env.device).cuda_stream)
@@ -278,20 +302,24 @@ class Algo_PPO:
 
     def _step_pair(self, actor, critic, opti_actor, opti_critic, n=None, row=None):
         """All-reduce the pair's packed gradients (one collective) and take both Adam steps in one launch (PY:810-815); with
-        target_kl, the launch that halts the pair on the device (its step counts are settled after the update, _diag_finish)."""
+        target_kl, the launch that halts the pair on the device (its step counts are settled after the update, _diag_finish); with
+        max_grad_norm, the launch that clips each net's gradient first (inside update() it also records the two norms)."""
         allreduce_sum_(self._gbuf[id(actor)])
         actor.step += 1; critic.step += 1
+        L = _lib.lib()
+        adam = (actor.flat.data_ptr(), actor.grad.data_ptr(), actor.m.data_ptr(), actor.v.data_ptr(), actor.n_param, opti_actor.lr, actor.step,
+                critic.flat.data_ptr(), critic.grad.data_ptr(), critic.m.data_ptr(), critic.v.data_ptr(), critic.n_param, opti_critic.lr,
+                critic.step, 0.9, 0.999, 1e-8)
+        halt = None
         if row is not None and self.target_kl is not None:
-            p = self._rec_pair
-            check(_lib.lib().mhppo_adam2_halt(actor.flat.data_ptr(), actor.grad.data_ptr(), actor.m.data_ptr(), actor.v.data_ptr(), actor.n_param,
-                                              opti_actor.lr, actor.step, critic.flat.data_ptr(), critic.grad.data_ptr(), critic.m.data_ptr(),
-                                              critic.v.data_ptr(), critic.n_param, opti_critic.lr, critic.step, 0.9, 0.999, 1e-8,
-                                              self._klslot[id(actor)].data_ptr(), 1.5 * float(self.target_kl) * n,
-                                              self._halt.data_ptr() + 4 * p, row, self._stream()))
-            return
-        check(_lib.lib().mhppo_adam2(actor.flat.data_ptr(), actor.grad.data_ptr(), actor.m.data_ptr(), actor.v.data_ptr(), actor.n_param,
-                                     opti_actor.lr, actor.step, critic.flat.data_ptr(), critic.grad.data_ptr(), critic.m.data_ptr(),
-                                     critic.v.data_ptr(), critic.n_param, opti_critic.lr, critic.step, 0.9, 0.999, 1e-8, self._stream()))
+            halt = (self._klslot[id(actor)].data_ptr(), 1.5 * float(self.target_kl) * n, self._halt.data_ptr() + 4 * self._rec_pair, row)
+        if self.max_grad_norm is not None:
+            norms = None if self._norms is None else self._norms.data_ptr() + 16 * self._rec_i
+            check(L.mhppo_adam2_clip(*adam, float(self.max_grad_norm), norms, *(halt or (None, 0.0, None, None)), self._stream()))
+        elif halt is not None:
+            check(L.mhppo_adam2_halt(*adam, *halt, self._stream()))
+        else:
+            check(L.mhppo_adam2(*adam, self._stream()))
 
     # -- one epoch of train_model_d (PY:818-851) on the choice buffer -------------------------------------------
     def train_model_d(self, actor, critic, opti_actor, opti_critic):
@@ -352,8 +380,9 @@ class Algo_PPO:
         self.rollout.futur_rewards()                    # also the choice reward rew_d, which GAE mode uses too
         if self.gae_lambda is not None:
             self._prepare_gae()
-        if self._diag:
-            self._diag_begin(epochs)
+        clip = self.max_grad_norm is not None
+        if self._diag or clip:
+            self._steps_begin(epochs, clip)
         try:
             if self.n_minibatches is not None:
                 self._update_minibatches(epochs)
@@ -366,64 +395,72 @@ class Algo_PPO:
                     self._pos = (e, 0)
                     self.train_model_d(self.actor_net_choice, self.critic_net_choice, self.optimizer_actor_choice, self.optimizer_critic_choice)
             pending = self._diag_fetch() if self._diag else None
+            pending_norms = _to_host_async(self._norms[:self._n_steps]) if clip else None
         finally:
-            self._rec = None                             # train_model_c / _d outside update() take the plain path
-        failed = _lib.lib().mhppo_tc_failures()          # (synchronises the device: the record's copy has landed with it)
+            self._steps_done, self._steps = self._steps, None
+            self._rec = self._norms = None               # train_model_c / _d outside update() take the plain path
+        failed = _lib.lib().mhppo_tc_failures()          # (synchronises the device: the copies have landed with it)
         if pending is not None:
             host, done = pending
             done.synchronize()
             self._diag_finish(host.numpy())              # step counts settled even when the update is reported broken below
+        if pending_norms is not None:
+            host, done = pending_norms
+            done.synchronize()
+            self._grad_norms_finish(host.numpy())
         if failed:                                       # a tensor-core kernel gave up waiting for its MMAs: its gradients are garbage
             raise RuntimeError("a tcgen05 kernel of the update timed out on its mbarrier; the parameters of this update are not "
                                "trustworthy (reload a checkpoint; MHPPO_MLP=ffma selects the CUDA-core kernels)")
 
-    # -- diagnostics (diagnostics=True / target_kl) ---------------------------------------------------------------------
-    def _diag_begin(self, epochs):
-        """A zeroed record of one fp64 row per possible step of this update, the pairs' halt flags cleared."""
+    # -- per-step records of an update: diagnostics (diagnostics=True / target_kl) and gradient norms (max_grad_norm) ----------
+    def _steps_begin(self, epochs, clip):
+        """The step bookkeeping of this update; with diagnostics a zeroed record of one fp64 row per possible step and the pairs'
+        halt flags cleared, with clipping one fp64 (actor, critic) norm row per possible step.  Both are indexed by the same step
+        counter, so their rows line up."""
         B = int(self.n_minibatches) if self.n_minibatches is not None else 1
-        self._rec = torch.zeros(3 * epochs * B, DIAG_ROW, dtype=torch.float64, device=self._stats.device)
-        self._rec_steps = {p: [] for p in PAIRS}        # per pair: (epoch, minibatch, n, record row), in launch order
-        self._rec_used = 0
-        self._rec_steps0 = {p: (a.step, c.step) for p, a, c in self._pair_nets()}
+        dev = self._stats.device
+        self._steps = {p: [] for p in PAIRS}             # per pair: (epoch, minibatch, n, step index), in launch order
+        self._n_steps = 0
         self._pos = (0, 0)
-        if self.target_kl is not None:
-            self._halt.zero_()
+        if self._diag:
+            self._rec = torch.zeros(3 * epochs * B, DIAG_ROW, dtype=torch.float64, device=dev)
+            self._rec_steps0 = {p: (a.step, c.step) for p, a, c in self._pair_nets()}
+            if self.target_kl is not None:
+                self._halt.zero_()
+        if clip:
+            self._norms = torch.zeros(3 * epochs * B, 2, dtype=torch.float64, device=dev)
 
     def _pair_nets(self):
         return (("cross", self.actor_net_cross, self.critic_net_cross), ("wait", self.actor_net_wait, self.critic_net_wait),
                 ("choice", self.actor_net_choice, self.critic_net_choice))
 
     def _diag_row(self, pair, n):
-        """Device address of the next record row for a step of pair 0 / 1 / 2 with n samples over all ranks; None outside update()
-        or without diagnostics."""
-        if self._rec is None:
+        """Counts a step of pair 0 / 1 / 2 with n samples over all ranks (inside update(), with diagnostics or clipping) and returns
+        the device address of its record row; None outside update() or without diagnostics."""
+        if self._steps is None:
             return None
-        i = self._rec_used
-        self._rec_used += 1
-        self._rec_steps[PAIRS[pair]].append((self._pos[0], self._pos[1], int(n), i))
-        self._rec_pair = pair
-        return self._rec.data_ptr() + 8 * DIAG_ROW * i
+        i = self._n_steps
+        self._n_steps += 1
+        self._steps[PAIRS[pair]].append((self._pos[0], self._pos[1], int(n), i))
+        self._rec_pair, self._rec_i = pair, i
+        return None if self._rec is None else self._rec.data_ptr() + 8 * DIAG_ROW * i
 
     def _diag_fetch(self):
         """One all-reduce of the record's sums over the ranks (the taken flags are the same on every rank) and one asynchronous
         device-to-host copy of the used rows into pinned memory; returns (host tensor, event of the copy).  The host waits for it
         in the same synchronisation as the mhppo_tc_failures copy that ends every update."""
-        used = self._rec_used
+        used = self._n_steps
         if _dist() is not None and used:
             s = self._rec[:used, :DIAG_ROW - 1].contiguous()
             allreduce_sum_(s)
             self._rec[:used, :DIAG_ROW - 1] = s
-        host = torch.empty((used, DIAG_ROW), dtype=torch.float64, pin_memory=True)
-        host.copy_(self._rec[:used], non_blocking=True)
-        done = torch.cuda.Event()
-        done.record(torch.cuda.current_stream(self._rec.device))
-        return host, done
+        return _to_host_async(self._rec[:used])
 
     def _diag_finish(self, host):
         """last_update_stats from the copied record; with target_kl, each pair's Adam step counts become the steps it took."""
         out = {}
         for p, actor, critic in self._pair_nets():
-            steps = self._rec_steps[p]
+            steps = self._steps_done[p]
             a = np.zeros(len(steps), dtype=DIAG_FIELDS)
             for j, (e, b, n, i) in enumerate(steps):
                 a[j]["epoch"], a[j]["minibatch"], a[j]["n"] = e, b, n
@@ -435,6 +472,24 @@ class Algo_PPO:
                 s0a, s0c = self._rec_steps0[p]
                 actor.step, critic.step = s0a + int(a["taken"].sum()), s0c + int(a["taken"].sum())
         self.last_update_stats = out
+
+    def _grad_norms_finish(self, host):
+        """last_grad_norms from the copied norms (the same on every rank: they are taken after the gradient all-reduce)."""
+        out = {}
+        for p in PAIRS:
+            steps = self._steps_done[p]
+            a = np.zeros(len(steps), dtype=GRAD_NORM_FIELDS)
+            for j, (e, b, n, i) in enumerate(steps):
+                a[j]["epoch"], a[j]["minibatch"] = e, b
+                a[j]["actor_grad_norm"], a[j]["critic_grad_norm"] = host[i]
+            out[p] = a
+        self.last_grad_norms = out
+
+    def grad_norms_summary(self):
+        """Per pair: the means of last_grad_norms' actor and critic norms over the launched steps, and the steps launched."""
+        return {p: dict(actor_grad_norm=float(np.mean(a["actor_grad_norm"])) if len(a) else float("nan"),
+                        critic_grad_norm=float(np.mean(a["critic_grad_norm"])) if len(a) else float("nan"), steps_launched=int(len(a)))
+                for p, a in self.last_grad_norms.items()}
 
     def diagnostics_summary(self):
         """Per pair: the means of last_update_stats' float fields over the launched steps, and the steps launched / taken."""
@@ -513,6 +568,8 @@ class Algo_PPO:
             self.ep_scenario_balance.append([nc, nw])
             if self._diag:
                 self.ep_diagnostics.append(self.diagnostics_summary())
+            if self.max_grad_norm is not None:
+                self.ep_grad_norms.append(self.grad_norms_summary())
             self.total_loop += 1
             if verbose:
                 print("Episode * {} * cross {:.4f} wait {:.4f} choice {:.4f}  (#cross {} #wait {})".format(
