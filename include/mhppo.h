@@ -341,6 +341,24 @@ int mhppo_adam2_clip(float *p0_dev, const float *g0_dev, float *m0_dev, float *v
                      float eps, double max_norm, double *norms_out_dev, const float *kl_sum_dev, double kl_limit, int32_t *halt_dev,
                      double *record_row_dev, void *stream);
 
+/* mhppo_adam2_clip with the KL-adaptive learning rate (an option, Algo_PPO(lr_schedule="adaptive", desired_kl=delta); rsl_rl's
+ * schedule="adaptive" rule, decided on the device before the step): kl = *kl_sum_dev / n, the pair's all-reduced actor k3 sum (the
+ * fp32 slot mhppo_ppo_grad_diag writes behind the pair's packed gradients) over the step's sample count n; then on each net's fp32 lr
+ * state lr_dev[0] (actor, net 0) and lr_dev[1] (critic, net 1) separately:
+ *   kl > 2 delta            lr = max(1e-5, lr / 1.5)
+ *   0 < kl < delta / 2      lr = min(1e-2, lr * 1.5)
+ *   otherwise (NaN, +-inf)  lr unchanged
+ * each change computed in fp64 and rounded to fp32.  The step uses that lr: step size (float)((double)lr / (1 - beta1^step)), the
+ * formula of mhppo_adam2, so a step whose lr did not change is mhppo_adam2_clip's (mhppo_adam2's when nothing is clipped) bit for bit.
+ * lr0 and lr1 are unused.  lrs_out_dev (may be NULL): fp64 [2], the lrs the step used.  With the halt (kl_sum, halt_dev, record_row_dev)
+ * its test comes first: a halted step changes neither the weights nor lr_dev nor lrs_out_dev.  max_norm = +inf: no clipping.  One launch.
+ * MHPPO_EINVAL: mhppo_adam2_clip's checks, lr_dev or kl_sum_dev NULL, desired_kl NaN or <= 0, n NaN or <= 0. */
+int mhppo_adam2_sched(float *p0_dev, const float *g0_dev, float *m0_dev, float *v0_dev, int32_t n0, float lr0, int32_t step0, float *p1_dev,
+                      const float *g1_dev, float *m1_dev, float *v1_dev, int32_t n1, float lr1, int32_t step1, float beta1, float beta2,
+                      float eps, double max_norm, double *norms_out_dev, const float *halt_kl_sum_dev, double kl_limit, int32_t *halt_dev,
+                      double *record_row_dev, float *lr_dev, const float *kl_sum_dev, double n, double desired_kl, double *lrs_out_dev,
+                      void *stream);
+
 /* Self-test of the tcgen05 / TMEM building blocks behind the policy GEMMs: D[128,N] = A[128,K] * B[N,K]^T on one CTA,
  * mode 0 = one tf32 pass, mode 1 = 3xTF32 split accumulation.  (N,K) in {(64,32),(32,64),(64,16),(16,32)}. */
 /* implementation of the 13-input nets' kernels: 0 auto (tcgen05 for the update: forward + backward-data of ppo_grad /

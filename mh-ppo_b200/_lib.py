@@ -87,6 +87,9 @@ SYMBOLS = {
                          + [C.c_float] * 3 + [C.c_void_p, C.c_double] + [C.c_void_p] * 3),
     "mhppo_adam2_clip": (C.c_int, [C.c_void_p] * 4 + [C.c_int32, C.c_float, C.c_int32] + [C.c_void_p] * 4 + [C.c_int32, C.c_float, C.c_int32]
                          + [C.c_float] * 3 + [C.c_double, C.c_void_p, C.c_void_p, C.c_double] + [C.c_void_p] * 3),
+    "mhppo_adam2_sched": (C.c_int, [C.c_void_p] * 4 + [C.c_int32, C.c_float, C.c_int32] + [C.c_void_p] * 4 + [C.c_int32, C.c_float, C.c_int32]
+                          + [C.c_float] * 3 + [C.c_double, C.c_void_p, C.c_void_p, C.c_double] + [C.c_void_p] * 2
+                          + [C.c_void_p, C.c_void_p, C.c_double, C.c_double, C.c_void_p, C.c_void_p]),
     "mhppo_tc_failures": (C.c_int, []),
     "mhppo_set_mlp_mode": (C.c_int, [C.c_int32]),
     "mhppo_set_gaussian_head": (C.c_int, [C.c_float, C.c_float, C.c_float, C.c_float]),

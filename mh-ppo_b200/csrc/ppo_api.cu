@@ -551,4 +551,36 @@ int mhppo_adam2_clip(float *p0, const float *g0, float *m0, float *v0, int32_t n
     return ck(cudaGetLastError(), "k_adam2_clip");
 }
 
+int mhppo_adam2_sched(float *p0, const float *g0, float *m0, float *v0, int32_t n0, float lr0, int32_t step0, float *p1, const float *g1,
+                      float *m1, float *v1, int32_t n1, float lr1, int32_t step1, float beta1, float beta2, float eps, double max_norm,
+                      double *norms_out, const float *kl_sum, double kl_limit, int32_t *halt, double *record_row, float *lr_dev,
+                      const float *kl_sum_dev, double n, double desired_kl, double *lrs_out_dev, void *stream) {
+    if (!p0 || !g0 || !m0 || !v0 || !p1 || !g1 || !m1 || !v1 || n0 <= 0 || n1 <= 0 || step0 < 1 || step1 < 1) return api_fail(MHPPO_EINVAL, "bad argument");
+    if (!(max_norm > 0.0)) return api_fail(MHPPO_EINVAL, "max_norm must be > 0 (+inf: no clipping)");
+    const int nhalt = (kl_sum != nullptr) + (halt != nullptr) + (record_row != nullptr);
+    if (nhalt != 0 && nhalt != 3) return api_fail(MHPPO_EINVAL, "kl_sum, halt and record_row go together (all null: no halt)");
+    if (nhalt && std::isnan(kl_limit)) return api_fail(MHPPO_EINVAL, "kl_limit must not be NaN");
+    if (!lr_dev || !kl_sum_dev) return api_fail(MHPPO_EINVAL, "null argument");
+    if (!(desired_kl > 0.0)) return api_fail(MHPPO_EINVAL, "desired_kl must be > 0");
+    if (!(n > 0.0)) return api_fail(MHPPO_EINVAL, "n must be > 0");
+    auto mk = [&](float *p, const float *g, float *m, float *v, int n, float lr, int step) {
+        const double bc1 = 1.0 - std::pow((double)beta1, (double)step), bc2 = 1.0 - std::pow((double)beta2, (double)step);
+        AdamArgs a; a.p = p; a.g = g; a.m = m; a.v = v; a.n = n; a.step_size = (float)((double)lr / bc1); a.inv_sqrt_bc2 = (float)(1.0 / std::sqrt(bc2));
+        return a;
+    };
+    AdaptArgs ad;
+    ad.lr = lr_dev; ad.kl_sum = kl_sum_dev; ad.lrs_out = lrs_out_dev; ad.n = n; ad.desired_kl = desired_kl;
+    ad.bc1[0] = 1.0 - std::pow((double)beta1, (double)step0);
+    ad.bc1[1] = 1.0 - std::pow((double)beta1, (double)step1);
+    const AdamArgs a0 = mk(p0, g0, m0, v0, n0, lr0, step0), a1 = mk(p1, g1, m1, v1, n1, lr1, step1);
+    if (nhalt)
+        k_adam2_clip<true, true><<<dim3(1, 2), kClipBlock, 0, (cudaStream_t)stream>>>(a0, a1, beta1, beta2, eps, max_norm, norms_out, kl_sum,
+                                                                                      kl_limit, (int *)halt, record_row + 9, ad);
+    else
+        k_adam2_clip<false, true><<<dim3(1, 2), kClipBlock, 0, (cudaStream_t)stream>>>(a0, a1, beta1, beta2, eps, max_norm, norms_out,
+                                                                                       nullptr, 0.0, nullptr, nullptr, ad);
+    api_count_launch();
+    return ck(cudaGetLastError(), "k_adam2_clip");
+}
+
 }  // extern "C"

@@ -799,13 +799,22 @@ __global__ void __launch_bounds__(256) k_adam2_halt(AdamArgs a0, AdamArgs a1, fl
 // warp 0 over the warp sums: a fixed order, repeatable bit for bit), pass 2 is k_adam2's element arithmetic on g * coef (exact
 // for coef = 1, so an unclipped step is k_adam2's bit for bit).  g is not written.  norms_out[y] = norm when norms_out != NULL.
 // HALT: k_adam2_halt's halt on top, tested after the norms are written, so a step the halt skips still reports its norm.
+// ADAPT: the KL-adaptive learning rate (Algo_PPO(lr_schedule="adaptive")), see AdaptArgs; a.step_size is then ignored.
 constexpr int kClipBlock = 1024;
-template <bool HALT>
+
+// rsl_rl's adaptive rule on each net's fp32 lr state lr[y], decided by thread 0 of net y's CTA after the halt test: kl = *kl_sum / n
+// (the pair's all-reduced actor k3 sum over the step's n samples);
+// kl > 2 delta: lr = max(1e-5, lr / 1.5); else 0 < kl < delta / 2: lr = min(1e-2, lr * 1.5); otherwise (NaN, +-inf included) the
+// lr stays.  Each change is computed in fp64 and rounded to fp32; the step then uses step_size = (float)((double)lr / bc1[y]), the
+// host's formula, so a step whose lr did not change is k_adam2's bit for bit.  lrs_out[y] (may be NULL) = the lr the step used.
+struct AdaptArgs { float *lr; const float *kl_sum; double *lrs_out; double n, desired_kl, bc1[2]; };
+
+template <bool HALT, bool ADAPT = false>
 __global__ void __launch_bounds__(kClipBlock) k_adam2_clip(AdamArgs a0, AdamArgs a1, float beta1, float beta2, float eps, double max_norm,
                                                            double *__restrict__ norms_out, const float *__restrict__ kl_sum,
-                                                           double kl_limit, int *halt, double *taken) {
+                                                           double kl_limit, int *halt, double *taken, AdaptArgs ad = AdaptArgs{}) {
     __shared__ double wsum[kClipBlock / 32];
-    __shared__ float coef_s;
+    __shared__ float coef_s, step_s;
     const AdamArgs a = blockIdx.y ? a1 : a0;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     double ss = 0.0;
@@ -828,13 +837,27 @@ __global__ void __launch_bounds__(kClipBlock) k_adam2_clip(AdamArgs a0, AdamArgs
         if ((double)*kl_sum > kl_limit) { if (threadIdx.x == 0) *(volatile int *)halt = 1; return; }
         if (blockIdx.y == 0 && threadIdx.x == 0) *taken = 1.0;
     }
-    const float coef = coef_s;
+    if (ADAPT) {
+        if (threadIdx.x == 0) {
+            const double kl = (double)*ad.kl_sum / ad.n;
+            float lr = ad.lr[blockIdx.y];
+            if (isfinite(kl)) {
+                if (kl > 2.0 * ad.desired_kl) lr = (float)fmax(1e-5, (double)lr / 1.5);
+                else if (kl > 0.0 && kl < 0.5 * ad.desired_kl) lr = (float)fmin(1e-2, (double)lr * 1.5);
+            }
+            ad.lr[blockIdx.y] = lr;
+            if (ad.lrs_out) ad.lrs_out[blockIdx.y] = (double)lr;
+            step_s = (float)((double)lr / (blockIdx.y ? ad.bc1[1] : ad.bc1[0]));
+        }
+        __syncthreads();
+    }
+    const float coef = coef_s, step_size = ADAPT ? step_s : a.step_size;
     for (int i = threadIdx.x; i < a.n; i += kClipBlock) {
         const float gi = a.g[i] * coef;
         const float mi = beta1 * a.m[i] + (1.0f - beta1) * gi;
         const float vi = beta2 * a.v[i] + (1.0f - beta2) * gi * gi;
         a.m[i] = mi; a.v[i] = vi;
-        a.p[i] = a.p[i] - a.step_size * (mi / (sqrtf(vi) * a.inv_sqrt_bc2 + eps));
+        a.p[i] = a.p[i] - step_size * (mi / (sqrtf(vi) * a.inv_sqrt_bc2 + eps));
     }
 }
 

@@ -25,6 +25,25 @@ One more, also off by default (DESIGN.md §5 "Gradient-norm clipping"):
                       A non-finite norm leaves the step unclipped; g = inf never clips.  Fused into the pair's Adam launch
                       (mhppo_adam2_clip).  update() leaves every step's two norms in `last_grad_norms`, train() appends
                       per-iteration means to `ep_grad_norms`.
+A learning-rate schedule, also off by default (DESIGN.md §4 "Learning-rate schedules", §5 "Learning-rate schedule cost"):
+  lr_schedule=None    every lr stays what its Adam holds (the constructor's actor_lr / critic_lr / actor_d_lr / critic_d_lr).
+  "linear"            with lr_anneal_iterations=K (an integer >= 1): at the start of every update() each of the six optimisers gets
+                      lr = lr0 * max(0, 1 - k / K), lr0 its constructor value and k = self.total_loop, the iterations train() has
+                      completed (loading() sets it too); CleanRL's anneal_lr.  Host only: the steps take the usual Adam launches.
+  "adaptive"          with desired_kl=delta (a finite number > 0): rsl_rl's schedule="adaptive" rule, decided on the device before
+                      every step of a pair (each full-batch epoch, each minibatch that takes a step): kl = the step's approx. KL (the
+                      all-reduced k3 sum over its n samples, the estimator of the diagnostics; not rsl_rl's analytic Gaussian KL,
+                      which needs the old means the rollout does not keep); kl > 2 delta: lr = max(1e-5, lr / 1.5); 0 < kl < delta / 2:
+                      lr = min(1e-2, lr * 1.5); otherwise (NaN and inf included) unchanged.  Each of the pair's two nets applies the
+                      rule to its own lr with the pair's one kl.  The lr state is fp32 on the device (changes computed in fp64 and
+                      rounded); it is loaded from the six Adam.lr at the start of each update and written back to them in the
+                      synchronisation that ends it, so it carries over between updates and a value set between updates is honoured.
+                      Turns the diagnostics on.  With target_kl the halt test comes first (a halted step changes no weight and no
+                      lr); with max_grad_norm the gradient is clipped, then the step takes the adapted lr.  One launch per step
+                      (mhppo_adam2_sched).  train_model_c / _d called outside update() take the plain path with Adam.lr.
+  update() leaves the lr of every step (fp32 values; NaN for a step the target-KL halt skipped in "adaptive" mode) in `last_lrs`,
+  train() appends each pair's lrs after the update to `ep_lrs`.  Checkpoints keep no lr: a resumed "adaptive" run restarts from
+  the constructor's values.
 
 One iteration = one 80-step episode in every env of the vectorised env.  Multi-GPU: one process per GPU, envs
 sharded per rank; the only collectives are the all-reduce of the three advantage statistics and of the flat
@@ -53,6 +72,8 @@ DIAG_FIELDS = [("epoch", np.int32), ("minibatch", np.int32), ("n", np.int64), ("
                ("approx_kl", np.float64), ("clip_fraction", np.float64), ("entropy", np.float64), ("explained_variance", np.float64),
                ("taken", np.bool_)]
 GRAD_NORM_FIELDS = [("epoch", np.int32), ("minibatch", np.int32), ("actor_grad_norm", np.float64), ("critic_grad_norm", np.float64)]
+LR_FIELDS = [("epoch", np.int32), ("minibatch", np.int32), ("actor_lr", np.float64), ("critic_lr", np.float64)]
+LR_SCHEDULES = ("linear", "adaptive")
 
 
 def diag_ratios(sums, n, choice):
@@ -137,13 +158,19 @@ class Algo_PPO:
         nbytes = max(L.mhppo_update_workspace_bytes(self.num_states_c), L.mhppo_update_workspace_bytes(self.num_states_d))
         self._ws = torch.zeros(nbytes, dtype=torch.uint8, device=dev)
         self._stats = torch.zeros(3, dtype=torch.float64, device=dev)
-        self._diag = bool(self.diagnostics) or self.target_kl is not None
+        self._diag = bool(self.diagnostics) or self.target_kl is not None or self.lr_schedule == "adaptive"
         self._steps = None                                # per pair, the steps of the update in progress (diagnostics, clipping)
         self._rec = None                                  # the record of the update in progress (diagnostics)
         self._norms = None                                # its gradient norms, fp64 [step][actor, critic] (clipping)
         self._halt = torch.zeros(3, dtype=torch.int32, device=dev)
         self.last_update_stats, self.ep_diagnostics = {}, []
         self.last_grad_norms, self.ep_grad_norms = {}, []
+        self._lr0 = [(oa.lr, oc.lr) for _, (oa, oc) in self._pair_optimizers()]          # the constructor's lrs ("linear")
+        self._lrs = None                                  # the lrs of the update in progress, fp64 [step][actor, critic] ("adaptive")
+        if self.lr_schedule == "adaptive":               # the lr state, fp32 [pair][actor, critic], and its pinned staging copy
+            self._lr_dev = torch.zeros(len(PAIRS), 2, dtype=torch.float32, device=dev)
+            self._lr_host = torch.zeros(len(PAIRS), 2, dtype=torch.float32, pin_memory=True)
+        self.last_lrs, self.ep_lrs = {}, []
         self._loss = torch.zeros(2, dtype=torch.float64, device=dev)
         self.last_losses = {}
         self._sel_cache = {}
@@ -182,6 +209,7 @@ class Algo_PPO:
         self.n_minibatches = None
         self.diagnostics, self.target_kl = False, None
         self.max_grad_norm = None
+        self.lr_schedule, self.desired_kl, self.lr_anneal_iterations = None, None, None
         for k, v in hyperparameters.items():
             setattr(self, k, v)
 
@@ -206,6 +234,19 @@ class Algo_PPO:
         g = self.max_grad_norm
         if g is not None and not (real(g) and float(g) > 0.0):
             raise ValueError("max_grad_norm must be None or a number > 0 (inf: record the norms, never clip), got %r" % (g,))
+        s, d, K = self.lr_schedule, self.desired_kl, self.lr_anneal_iterations
+        if not (s is None or (isinstance(s, str) and s in LR_SCHEDULES)):
+            raise ValueError("lr_schedule must be None, 'linear' or 'adaptive', got %r" % (s,))
+        if s == "adaptive":
+            if not (real(d) and math.isfinite(float(d)) and float(d) > 0.0):
+                raise ValueError("lr_schedule='adaptive' needs desired_kl, a finite number > 0, got %r" % (d,))
+        elif d is not None:
+            raise ValueError("desired_kl is an option of lr_schedule='adaptive', got %r with lr_schedule=%r" % (d, s))
+        if s == "linear":
+            if not (isinstance(K, numbers.Integral) and not isinstance(K, bool) and int(K) >= 1):
+                raise ValueError("lr_schedule='linear' needs lr_anneal_iterations, an integer >= 1, got %r" % (K,))
+        elif K is not None:
+            raise ValueError("lr_anneal_iterations is an option of lr_schedule='linear', got %r with lr_schedule=%r" % (K, s))
 
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.env.device).cuda_stream)
@@ -303,7 +344,8 @@ class Algo_PPO:
     def _step_pair(self, actor, critic, opti_actor, opti_critic, n=None, row=None):
         """All-reduce the pair's packed gradients (one collective) and take both Adam steps in one launch (PY:810-815); with
         target_kl, the launch that halts the pair on the device (its step counts are settled after the update, _diag_finish); with
-        max_grad_norm, the launch that clips each net's gradient first (inside update() it also records the two norms)."""
+        max_grad_norm, the launch that clips each net's gradient first (inside update() it also records the two norms); inside an
+        update with lr_schedule="adaptive", the launch that first adapts the pair's two lrs on the device (mhppo_adam2_sched)."""
         allreduce_sum_(self._gbuf[id(actor)])
         actor.step += 1; critic.step += 1
         L = _lib.lib()
@@ -313,8 +355,13 @@ class Algo_PPO:
         halt = None
         if row is not None and self.target_kl is not None:
             halt = (self._klslot[id(actor)].data_ptr(), 1.5 * float(self.target_kl) * n, self._halt.data_ptr() + 4 * self._rec_pair, row)
-        if self.max_grad_norm is not None:
-            norms = None if self._norms is None else self._norms.data_ptr() + 16 * self._rec_i
+        norms = None if self._norms is None else self._norms.data_ptr() + 16 * self._rec_i
+        if self._lrs is not None:
+            g = math.inf if self.max_grad_norm is None else float(self.max_grad_norm)
+            check(L.mhppo_adam2_sched(*adam, g, norms, *(halt or (None, 0.0, None, None)), self._lr_dev.data_ptr() + 8 * self._rec_pair,
+                                      self._klslot[id(actor)].data_ptr(), float(n), float(self.desired_kl),
+                                      self._lrs.data_ptr() + 16 * self._rec_i, self._stream()))
+        elif self.max_grad_norm is not None:
             check(L.mhppo_adam2_clip(*adam, float(self.max_grad_norm), norms, *(halt or (None, 0.0, None, None)), self._stream()))
         elif halt is not None:
             check(L.mhppo_adam2_halt(*adam, *halt, self._stream()))
@@ -380,8 +427,12 @@ class Algo_PPO:
         self.rollout.futur_rewards()                    # also the choice reward rew_d, which GAE mode uses too
         if self.gae_lambda is not None:
             self._prepare_gae()
-        clip = self.max_grad_norm is not None
-        if self._diag or clip:
+        clip, sched = self.max_grad_norm is not None, self.lr_schedule
+        if sched == "linear":
+            frac = max(0.0, 1.0 - self.total_loop / int(self.lr_anneal_iterations))
+            for (_, (oa, oc)), (la, lc) in zip(self._pair_optimizers(), self._lr0):
+                oa.lr, oc.lr = la * frac, lc * frac
+        if self._diag or clip or sched is not None:
             self._steps_begin(epochs, clip)
         try:
             if self.n_minibatches is not None:
@@ -396,9 +447,10 @@ class Algo_PPO:
                     self.train_model_d(self.actor_net_choice, self.critic_net_choice, self.optimizer_actor_choice, self.optimizer_critic_choice)
             pending = self._diag_fetch() if self._diag else None
             pending_norms = _to_host_async(self._norms[:self._n_steps]) if clip else None
+            pending_lrs = (_to_host_async(self._lrs[:self._n_steps]), _to_host_async(self._lr_dev)) if self._lrs is not None else None
         finally:
             self._steps_done, self._steps = self._steps, None
-            self._rec = self._norms = None               # train_model_c / _d outside update() take the plain path
+            self._rec = self._norms = self._lrs = None   # train_model_c / _d outside update() take the plain path
         failed = _lib.lib().mhppo_tc_failures()          # (synchronises the device: the copies have landed with it)
         if pending is not None:
             host, done = pending
@@ -408,6 +460,12 @@ class Algo_PPO:
             host, done = pending_norms
             done.synchronize()
             self._grad_norms_finish(host.numpy())
+        if pending_lrs is not None:
+            for _, done in pending_lrs:
+                done.synchronize()
+            self._lrs_finish(pending_lrs[0][0].numpy(), pending_lrs[1][0].numpy())
+        elif sched == "linear":
+            self._lrs_finish(None, None)
         if failed:                                       # a tensor-core kernel gave up waiting for its MMAs: its gradients are garbage
             raise RuntimeError("a tcgen05 kernel of the update timed out on its mbarrier; the parameters of this update are not "
                                "trustworthy (reload a checkpoint; MHPPO_MLP=ffma selects the CUDA-core kernels)")
@@ -429,6 +487,15 @@ class Algo_PPO:
                 self._halt.zero_()
         if clip:
             self._norms = torch.zeros(3 * epochs * B, 2, dtype=torch.float64, device=dev)
+        if self.lr_schedule == "adaptive":
+            # the lr state from the six Adam.lr (the previous update's synchronisation has ended every use of the staging copy)
+            self._lr_host.copy_(torch.tensor([[oa.lr, oc.lr] for _, (oa, oc) in self._pair_optimizers()], dtype=torch.float32))
+            self._lr_dev.copy_(self._lr_host, non_blocking=True)
+            self._lrs = torch.full((3 * epochs * B, 2), math.nan, dtype=torch.float64, device=dev)
+
+    def _pair_optimizers(self):
+        return (("cross", (self.optimizer_actor_cross, self.optimizer_critic_cross)), ("wait", (self.optimizer_actor_wait, self.optimizer_critic_wait)),
+                ("choice", (self.optimizer_actor_choice, self.optimizer_critic_choice)))
 
     def _pair_nets(self):
         return (("cross", self.actor_net_cross, self.critic_net_cross), ("wait", self.actor_net_wait, self.critic_net_wait),
@@ -484,6 +551,23 @@ class Algo_PPO:
                 a[j]["actor_grad_norm"], a[j]["critic_grad_norm"] = host[i]
             out[p] = a
         self.last_grad_norms = out
+
+    def _lrs_finish(self, rows, state):
+        """last_lrs: per pair and launched step the (actor, critic) lr the step used, fp32 values.  "adaptive": rows = the copied
+        per-step lrs (NaN where the target-KL halt skipped the step), state = the final device lr state, which the six Adam.lr take
+        over; "linear" (both None): every step used the Adam.lr set at the start of the update."""
+        if state is not None:
+            for (_, (oa, oc)), (la, lc) in zip(self._pair_optimizers(), state.tolist()):
+                oa.lr, oc.lr = la, lc
+        out = {}
+        for p, (oa, oc) in self._pair_optimizers():
+            steps = self._steps_done[p]
+            a = np.zeros(len(steps), dtype=LR_FIELDS)
+            for j, (e, b, n, i) in enumerate(steps):
+                a[j]["epoch"], a[j]["minibatch"] = e, b
+                a[j]["actor_lr"], a[j]["critic_lr"] = rows[i] if rows is not None else (np.float32(oa.lr), np.float32(oc.lr))
+            out[p] = a
+        self.last_lrs = out
 
     def grad_norms_summary(self):
         """Per pair: the means of last_grad_norms' actor and critic norms over the launched steps, and the steps launched."""
@@ -570,6 +654,8 @@ class Algo_PPO:
                 self.ep_diagnostics.append(self.diagnostics_summary())
             if self.max_grad_norm is not None:
                 self.ep_grad_norms.append(self.grad_norms_summary())
+            if self.lr_schedule is not None:
+                self.ep_lrs.append({p: dict(actor_lr=oa.lr, critic_lr=oc.lr) for p, (oa, oc) in self._pair_optimizers()})
             self.total_loop += 1
             if verbose:
                 print("Episode * {} * cross {:.4f} wait {:.4f} choice {:.4f}  (#cross {} #wait {})".format(

@@ -4,7 +4,10 @@
 
 Per entry: registers, stack frame / spill stores / spill loads (bytes).  A template parameter appended with a default keeps the
 old instance under a longer name (`k_ppo_grad<16, 0, false>` is now `k_ppo_grad<16, 0, false, false>`): a parent entry that is
-missing by name is matched to the new entry whose name is the parent's with `, (bool)0` (false) added to its template arguments."""
+missing by name is matched to the new entry whose name is the parent's with `, (bool)0` (false) added to its template arguments,
+and, failing that, to the one such entry whose parameter list starts with the parent's and goes on (a defaulted trailing kernel
+parameter that only the new instance reads: `k_adam2_clip<false>(..., double *)` is now `k_adam2_clip<false, false>(..., double *,
+mhppo::AdaptArgs)`)."""
 import re
 import subprocess
 import sys
@@ -52,6 +55,9 @@ def main(old_log, new_log):
         name = dn[k]
         alt = name.replace(">(", ", (bool)0>(", 1)
         nk = by_name_new.get(name) or by_name_new.get(alt)
+        if nk is None and alt.endswith(")"):
+            longer = [k2 for n2, k2 in by_name_new.items() if n2.startswith(alt[:-1] + ", ")]
+            nk = longer[0] if len(longer) == 1 else None
         if nk is None:
             missing.append(name)
             continue
@@ -68,7 +74,7 @@ def main(old_log, new_log):
         print("missing    %s" % name)
     renamed = sum(1 for nk, k in matched.items() if dn[nk] != dn[k])
     print("\n%d kernel entries of the parent build found in this build (%d of them under a name with the new defaulted template "
-          "parameter); %d with different registers, stack frame or spills; %d missing"
+          "parameter or trailing kernel parameter); %d with different registers, stack frame or spills; %d missing"
           % (len(matched), renamed, len(changed), len(missing)))
 
 
