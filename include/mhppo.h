@@ -260,6 +260,21 @@ int mhppo_ppo_grad_ent(int32_t n_in, int32_t head, const float *x_dev, int32_t D
  * mhppo_update_workspace_bytes is larger).  MHPPO_EINVAL for null pointers, T < 1, CN < 1, gamma or lambda outside [0, 1]. */
 int mhppo_gae(const float *rew_dev, const float *V_dev, const int8_t *route_dev, int32_t T, int64_t CN, double gamma, double lambda,
               float *ret_dev, double *stats6_dev, void *workspace_dev, void *stream);
+/* Reward normalisation (an option, Algo_PPO(normalize_reward=True), SB3's VecNormalize reward path; the reference regresses
+ * unnormalised returns).  Column m of route_dev int8 [CN] takes part when route[m] >= 0.  mhppo_reward_moments writes this rank's
+ * batch moments to moments6_dev (fp64): (n, sum g, sum g^2) of the continuous stream, g_t = gamma g_{t-1} + r_t over t = 0 .. T-1 of
+ * rew_dev [T][CN] (g_{-1} = 0, fp64 without contraction), n = T x the present columns; then (n, sum x, sum x^2) of the choice
+ * stream, x = rew_d_dev[m], n = the present columns.  Fixed summation order (bitwise repeatable); workspace_dev: 196 608 bytes, as
+ * for mhppo_gae.  mhppo_reward_normalize: with merge != 0 it first merges moments6_dev (all-reduced over the ranks) into the
+ * running state rms_dev fp64 [2][3] = (count, mean, var) of the continuous, then the choice stream, in place, by SB3's
+ * RunningMeanStd.update_from_moments (a stream with n = 0 keeps its state); then rew_out [T][CN] and rew_d_out [CN] get
+ * clip(r / sqrt(var + 1e-8), -clip, clip) in fp64 (correctly rounded), rounded to fp32 once, with each stream's var; no mean is
+ * subtracted; clip = +inf never clips.  One launch (merge = 0) or two.  MHPPO_EINVAL for null pointers, T < 1, CN < 1, gamma
+ * outside [0, 1], clip NaN or <= 0. */
+int mhppo_reward_moments(const float *rew_dev, const float *rew_d_dev, const int8_t *route_dev, int32_t T, int64_t CN, double gamma,
+                         double *moments6_dev, void *workspace_dev, void *stream);
+int mhppo_reward_normalize(const float *rew_dev, const float *rew_d_dev, int32_t T, int64_t CN, const double *moments6_dev,
+                           double *rms_dev, int32_t merge, double clip, float *rew_out_dev, float *rew_d_out_dev, void *stream);
 /* Minibatch plan of an update (an option, Algo_PPO(n_minibatches=B); the reference's update is full-batch, PY:866-882).
  * In epoch e (0 .. epochs-1) the (car, env) column m = car*N + n, global env id g = cfg->env_id0 + n, goes to bucket
  *   b = (x0 * B) >> 32,  x0 = word 0 of Philox4x32-10(counter = (e*C + car, 3 | iteration << 8, g_lo, g_hi), key = cfg->seed)

@@ -449,6 +449,44 @@ int mhppo_gae(const float *rew, const float *V, const int8_t *route, int32_t T, 
     return ck(cudaGetLastError(), "k_reduce_gae");
 }
 
+int mhppo_reward_moments(const float *rew, const float *rew_d, const int8_t *route, int32_t T, int64_t CN, double gamma, double *moments6,
+                         void *workspace, void *stream) {
+    if (!rew || !rew_d || !route || !moments6 || !workspace) return api_fail(MHPPO_EINVAL, "null argument");
+    if (T < 1 || CN < 1) return api_fail(MHPPO_EINVAL, "T and CN must be >= 1");
+    if (!(gamma >= 0.0 && gamma <= 1.0)) return api_fail(MHPPO_EINVAL, "gamma must lie in [0, 1]");
+    const int64_t blocks = (CN + kGaeBlock - 1) / kGaeBlock;
+    const int cap = 8 * sm_count() < kGaeGridMax ? 8 * sm_count() : kGaeGridMax;
+    const int grid = blocks < cap ? (int)blocks : cap;
+    double *partial = (double *)workspace;
+    cudaStream_t s = (cudaStream_t)stream;
+    k_reward_moments<<<grid, kGaeBlock, 0, s>>>(rew, rew_d, route, T, CN, gamma, partial);
+    api_count_launch();
+    int rc = ck(cudaGetLastError(), "k_reward_moments");
+    if (rc) return rc;
+    k_reduce_gae<<<1, 192, 0, s>>>(partial, grid, moments6);
+    api_count_launch();
+    return ck(cudaGetLastError(), "k_reduce_gae");
+}
+
+int mhppo_reward_normalize(const float *rew, const float *rew_d, int32_t T, int64_t CN, const double *moments6, double *rms, int32_t merge,
+                           double clip, float *rew_out, float *rew_d_out, void *stream) {
+    if (!rew || !rew_d || !moments6 || !rms || !rew_out || !rew_d_out) return api_fail(MHPPO_EINVAL, "null argument");
+    if (T < 1 || CN < 1) return api_fail(MHPPO_EINVAL, "T and CN must be >= 1");
+    if (!(clip > 0.0)) return api_fail(MHPPO_EINVAL, "clip must be > 0 (+inf: no clipping)");
+    const int64_t S = (int64_t)T * CN, tile = kScaleBlock * kScaleUnroll, blocks = (S + CN + tile - 1) / tile;
+    if (blocks > 0x7fffffff) return api_fail(MHPPO_EINVAL, "too many samples");
+    cudaStream_t s = (cudaStream_t)stream;
+    if (merge) {
+        k_reward_merge<<<1, 32, 0, s>>>(moments6, rms);
+        api_count_launch();
+        const int rc = ck(cudaGetLastError(), "k_reward_merge");
+        if (rc) return rc;
+    }
+    k_reward_scale<<<(unsigned)blocks, kScaleBlock, 0, s>>>(rew, rew_d, S, CN, rms, clip, rew_out, rew_d_out);
+    api_count_launch();
+    return ck(cudaGetLastError(), "k_reward_scale");
+}
+
 int mhppo_minibatch_plan(const mhppo_rollout_cfg *cfg, const int8_t *route, const int8_t *exist, const float *act_d, uint32_t iteration,
                          int32_t epochs, int32_t n_minibatches, int32_t *lists, int64_t *offsets, int64_t *counts, void *workspace,
                          void *stream) {

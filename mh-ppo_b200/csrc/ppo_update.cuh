@@ -621,6 +621,89 @@ __global__ void __launch_bounds__(192) k_reduce_gae(const double *__restrict__ p
     if (lane == 0) out[j] = acc;
 }
 
+// ---- reward normalisation (an option, Algo_PPO(normalize_reward=True); the reference regresses unnormalised returns) ---------
+// SB3's VecNormalize reward path with every (car, env) column as one env.  Two streams: the continuous rewards rew [T][CN] through
+// the forward running return g_t = gamma * g_{t-1} + r_t (g_{-1} = 0, fp64 without contraction), and the episodic choice rewards
+// rew_d [CN].  A column takes part when route[m] >= 0.
+// k_reward_moments: one thread per column m, k_gae's grid-stride shape; a forward scan with kGaeUnroll independent loads in flight,
+// coalesced over m; at most 64 registers, so that 4 CTAs per SM keep their loads in flight.  An absent column scans zeros (no
+// divergence in the warp) and adds nothing.  Per-CTA fp64 partials [grid][6] = (n, sum g, sum g^2) of the continuous stream, then
+// (n, sum x, sum x^2) of the choice stream; k_reduce_gae adds them in a fixed order (no atomics: repeated calls are bitwise identical).
+__global__ void __launch_bounds__(kGaeBlock, 4) k_reward_moments(const float *__restrict__ rew, const float *__restrict__ rew_d,
+                                                                 const int8_t *__restrict__ route, int T, int64_t CN, double gamma,
+                                                                 double *__restrict__ partial /* [grid][6] */) {
+    __shared__ double red[kGaeBlock / 32];
+    double st[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+    for (int64_t m = (int64_t)blockIdx.x * kGaeBlock + threadIdx.x; m < CN; m += (int64_t)gridDim.x * kGaeBlock) {
+        const bool on = route[m] >= 0;
+        double g = 0.0, sg = 0.0, sgg = 0.0;
+        for (int t0 = 0; t0 < T; t0 += kGaeUnroll) {
+            float rw[kGaeUnroll];
+#pragma unroll
+            for (int u = 0; u < kGaeUnroll; ++u) rw[u] = (on && t0 + u < T) ? rew[(int64_t)(t0 + u) * CN + m] : 0.f;
+#pragma unroll
+            for (int u = 0; u < kGaeUnroll; ++u) {
+                if (t0 + u >= T) break;
+                g = __dadd_rn(__dmul_rn(gamma, g), (double)rw[u]);
+                sg = __dadd_rn(sg, g);
+                sgg = __dadd_rn(sgg, __dmul_rn(g, g));
+            }
+        }
+        if (on) {
+            const double x = (double)rew_d[m];
+            st[0] += (double)T; st[1] += sg; st[2] += sgg;
+            st[3] += 1.0; st[4] += x; st[5] += x * x;
+        }
+    }
+#pragma unroll
+    for (int j = 0; j < 6; ++j) {
+        const double v = team_sum(st[j], red, threadIdx.x, kGaeBlock, 0);
+        if (threadIdx.x == 0) partial[(size_t)blockIdx.x * 6 + j] = v;
+    }
+}
+// one thread: merge the (all-reduced) batch moments into the running (count, mean, var) of each stream, rms [2][3], by SB3's
+// RunningMeanStd.update_from_moments; a stream whose batch is empty (n = 0) keeps its state
+__global__ void k_reward_merge(const double *__restrict__ moments, double *__restrict__ rms) {
+    if (threadIdx.x != 0) return;
+    for (int s = 0; s < 2; ++s) {
+        const double n = moments[3 * s];
+        if (!(n > 0.0)) continue;
+        const double mb = moments[3 * s + 1] / n, vb = fmax(moments[3 * s + 2] / n - mb * mb, 0.0);
+        double *st = rms + 3 * s;
+        const double count = st[0], mean = st[1], var = st[2];
+        const double delta = mb - mean, tot = count + n;
+        st[1] = mean + delta * n / tot;
+        st[2] = (var * count + vb * n + delta * delta * count * n / tot) / tot;
+        st[0] = tot;
+    }
+}
+// r~ = clip(r / sqrt(var + 1e-8), -clip, clip) in fp64 (correctly rounded division and sqrt), rounded to fp32 once; no mean is
+// subtracted (SB3).  Element i < S is rew[i] with the continuous stream's var, i >= S is rew_d[i - S] with the choice stream's.
+// Each thread loads kScaleUnroll elements, 256 apart (coalesced), before it scales any: independent loads in flight.
+// Comparisons rather than fmin / fmax, so a NaN reward stays NaN and clip = +inf never clips.
+constexpr int kScaleBlock = 256, kScaleUnroll = 8;
+__global__ void __launch_bounds__(kScaleBlock) k_reward_scale(const float *__restrict__ rew, const float *__restrict__ rew_d, int64_t S,
+                                                              int64_t M, const double *__restrict__ rms, double clip,
+                                                              float *__restrict__ rew_out, float *__restrict__ rew_d_out) {
+    const double sc = __dsqrt_rn(__dadd_rn(rms[2], 1e-8)), sd = __dsqrt_rn(__dadd_rn(rms[5], 1e-8));
+    const int64_t i0 = (int64_t)blockIdx.x * (kScaleBlock * kScaleUnroll) + threadIdx.x, n = S + M;
+    float r[kScaleUnroll];
+#pragma unroll
+    for (int u = 0; u < kScaleUnroll; ++u) {
+        const int64_t i = i0 + u * kScaleBlock;
+        r[u] = i < S ? rew[i] : (i < n ? rew_d[i - S] : 0.f);
+    }
+#pragma unroll
+    for (int u = 0; u < kScaleUnroll; ++u) {
+        const int64_t i = i0 + u * kScaleBlock;
+        if (i >= n) break;
+        const double x = __ddiv_rn((double)r[u], i < S ? sc : sd);
+        const float y = (float)(x < -clip ? -clip : (x > clip ? clip : x));
+        if (i < S) rew_out[i] = y;
+        else rew_d_out[i - S] = y;
+    }
+}
+
 // ---- minibatch plan (an option, Algo_PPO(n_minibatches=B); the reference's update is full-batch) --------------------------
 // In epoch e, column m = car*N + n (global env id g = env_id0 + n) goes to bucket
 //   b(car, g, e) = (w0 * B) >> 32,   w0 = word 0 of Philox4x32-10(counter = (e*C + car, 3 | iteration << 8, g_lo, g_hi), key = seed)

@@ -44,6 +44,19 @@ A learning-rate schedule, also off by default (DESIGN.md §4 "Learning-rate sche
   update() leaves the lr of every step (fp32 values; NaN for a step the target-KL halt skipped in "adaptive" mode) in `last_lrs`,
   train() appends each pair's lrs after the update to `ep_lrs`.  Checkpoints keep no lr: a resumed "adaptive" run restarts from
   the constructor's values.
+Reward normalisation, also off by default (DESIGN.md §4 "Reward normalisation", §5 "Reward normalisation"):
+  normalize_reward=False  True: SB3's VecNormalize reward path, each (car, env) column one env.  Once per rollout, at the start of
+                      update(), the batch moments of two streams -- the forward running return g_t = gamma * g_{t-1} + r_t of the `rew`
+                      buffer (cross / wait nets) and the episodic choice reward `rew_d` -- over the present columns (route >= 0) are
+                      all-reduced and merged into the running state `reward_rms` (device fp64 [2][3], rows continuous / choice,
+                      columns count / mean / var, starting at (1e-4, 0, 1)); every update then regresses on
+                      r~ = clip(r / sqrt(var + 1e-8), -c, c) (fp64, rounded to fp32 once; no mean subtracted) in place of the raw
+                      rewards: reward-to-go / GAE from r~, and r~_d as the choice critic's target and in its advantage.  A second
+                      update() on the same rollout rescales with the current state and does not merge again; a state set between
+                      updates is honoured.  The raw `rew`, `rl`, `rew_d` keep their values, so ep_reward_* stay raw.  update() leaves
+                      `last_reward_norm` = {"continuous", "choice"} -> dict(count, mean, var, scale), train() appends it to
+                      `ep_reward_norm`.  Checkpoints keep no statistics: a resumed run restarts them.
+  clip_reward=None    c > 0 (+inf: no clipping) with normalize_reward=True; None means 10.0 (SB3's default).
 
 One iteration = one 80-step episode in every env of the vectorised env.  Multi-GPU: one process per GPU, envs
 sharded per rank; the only collectives are the all-reduce of the three advantage statistics and of the flat
@@ -74,6 +87,8 @@ DIAG_FIELDS = [("epoch", np.int32), ("minibatch", np.int32), ("n", np.int64), ("
 GRAD_NORM_FIELDS = [("epoch", np.int32), ("minibatch", np.int32), ("actor_grad_norm", np.float64), ("critic_grad_norm", np.float64)]
 LR_FIELDS = [("epoch", np.int32), ("minibatch", np.int32), ("actor_lr", np.float64), ("critic_lr", np.float64)]
 LR_SCHEDULES = ("linear", "adaptive")
+REWARD_STREAMS = ("continuous", "choice")
+REWARD_RMS0 = ((1e-4, 0.0, 1.0), (1e-4, 0.0, 1.0))        # (count, mean, var) of each stream: SB3's RunningMeanStd(epsilon=1e-4)
 
 
 def diag_ratios(sums, n, choice):
@@ -171,6 +186,12 @@ class Algo_PPO:
             self._lr_dev = torch.zeros(len(PAIRS), 2, dtype=torch.float32, device=dev)
             self._lr_host = torch.zeros(len(PAIRS), 2, dtype=torch.float32, pin_memory=True)
         self.last_lrs, self.ep_lrs = {}, []
+        self.reward_rms = self._rn_moments = None            # reward normalisation: running state and this rollout's batch moments
+        if self.normalize_reward:
+            self.reward_rms = torch.tensor(REWARD_RMS0, dtype=torch.float64, device=dev)
+            self._rn_moments = torch.zeros(6, dtype=torch.float64, device=dev)
+        self._rn_iteration = None                            # the rollout whose batch reward_rms last merged
+        self.last_reward_norm, self.ep_reward_norm = {}, []
         self._loss = torch.zeros(2, dtype=torch.float64, device=dev)
         self.last_losses = {}
         self._sel_cache = {}
@@ -210,6 +231,7 @@ class Algo_PPO:
         self.diagnostics, self.target_kl = False, None
         self.max_grad_norm = None
         self.lr_schedule, self.desired_kl, self.lr_anneal_iterations = None, None, None
+        self.normalize_reward, self.clip_reward = False, None
         for k, v in hyperparameters.items():
             setattr(self, k, v)
 
@@ -247,6 +269,14 @@ class Algo_PPO:
                 raise ValueError("lr_schedule='linear' needs lr_anneal_iterations, an integer >= 1, got %r" % (K,))
         elif K is not None:
             raise ValueError("lr_anneal_iterations is an option of lr_schedule='linear', got %r with lr_schedule=%r" % (K, s))
+        if not isinstance(self.normalize_reward, bool):
+            raise ValueError("normalize_reward must be a bool, got %r" % (self.normalize_reward,))
+        c = self.clip_reward
+        if c is not None:
+            if not self.normalize_reward:
+                raise ValueError("clip_reward is an option of normalize_reward=True, got %r with normalize_reward=False" % (c,))
+            if not (real(c) and float(c) > 0.0):
+                raise ValueError("clip_reward must be None or a number > 0 (inf: no clipping), got %r" % (c,))
 
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.env.device).cuda_stream)
@@ -332,9 +362,35 @@ class Algo_PPO:
     def _prepare_gae(self):
         """GAE mode, once per update before the epochs: V_old of both critics, the returns and the advantage statistics of
         the cross and wait samples, all-reduced over the ranks once."""
-        _, stats6 = self.rollout.gae(self.critic_net_cross, self.critic_net_wait, self.gamma, self.gae_lambda,
-                                     selections=(self._selection(0), self._selection(1)), workspace=self._ws)
+        r = self.rollout
+        _, stats6 = r.gae(self.critic_net_cross, self.critic_net_wait, self.gamma, self.gae_lambda,
+                          selections=(self._selection(0), self._selection(1)), workspace=self._ws,
+                          rew=r.rew_n if self.normalize_reward else None)
         self._sel_cache["gae"] = allreduce_sum_(stats6)
+
+    def _normalize_rewards(self):
+        """Reward normalisation, once per update after the raw mhppo_returns (which forms rew_d): this rollout's batch moments of
+        both streams, all-reduced over the ranks (one device tensor, no host synchronisation), merged into reward_rms on the device
+        unless this rollout's batch is in it already; then r~ into rollout.rew_n / rew_dn and the reward-to-go from r~ (GAE mode
+        forms its returns from rew_n in _prepare_gae).  Returns the asynchronous host copy of reward_rms (host tensor, event)."""
+        r, L, st = self.rollout, _lib.lib(), self._stream()
+        rms = self.reward_rms
+        if not (isinstance(rms, torch.Tensor) and rms.dtype == torch.float64 and rms.shape == (2, 3) and rms.device == self._stats.device
+                and rms.is_contiguous()):
+            raise ValueError("reward_rms must be a contiguous float64 tensor of shape (2, 3) on %s" % (self._stats.device,))
+        if r.rew_n is None:
+            r.rew_n, r.rew_dn = torch.zeros_like(r.rew), torch.zeros_like(r.rew_d)
+        check(L.mhppo_reward_moments(r.rew.data_ptr(), r.rew_d.data_ptr(), r.route.data_ptr(), r.T, r.M, float(self.gamma),
+                                     self._rn_moments.data_ptr(), self._ws.data_ptr(), st))
+        allreduce_sum_(self._rn_moments)
+        merge = r.iteration != self._rn_iteration
+        self._rn_iteration = r.iteration
+        clip = 10.0 if self.clip_reward is None else float(self.clip_reward)
+        check(L.mhppo_reward_normalize(r.rew.data_ptr(), r.rew_d.data_ptr(), r.T, r.M, self._rn_moments.data_ptr(), rms.data_ptr(),
+                                       int(merge), clip, r.rew_n.data_ptr(), r.rew_dn.data_ptr(), st))
+        if self.gae_lambda is None:
+            r.futur_rewards(r.rew_n)
+        return _to_host_async(rms)
 
     def _gae_stats(self):
         if "gae" not in self._sel_cache:                    # train_model_c called outside update() on a new rollout
@@ -382,29 +438,30 @@ class Algo_PPO:
         ranks, fractions() = (f0, f1) of those n samples."""
         r, L, st = self.rollout, _lib.lib(), self._stream()
         ws, D = self._ws.data_ptr(), r.shape_env_d
+        rew_d = r.rew_dn if self.normalize_reward else r.rew_d       # the choice target: normalised (reward normalisation) or raw
         row = self._diag_row(2, n)
         if row is not None:
-            check(L.mhppo_critic_grad_diag(D, r.obs_d.data_ptr(), D, r.M, idx, K, r.M, critic.flat.data_ptr(), r.rew_d.data_ptr(), 1.0 / n,
+            check(L.mhppo_critic_grad_diag(D, r.obs_d.data_ptr(), D, r.M, idx, K, r.M, critic.flat.data_ptr(), rew_d.data_ptr(), 1.0 / n,
                                            critic.grad.data_ptr(), self._loss.data_ptr() + 8, r.V_d.data_ptr(), self._stats.data_ptr(), row, ws, st))
         else:
             check(L.mhppo_critic_grad_stats(D, r.obs_d.data_ptr(), D, r.M, idx, K, r.M, critic.flat.data_ptr(),
-                                            r.rew_d.data_ptr(), 1.0 / n, critic.grad.data_ptr(), self._loss.data_ptr() + 8,
+                                            rew_d.data_ptr(), 1.0 / n, critic.grad.data_ptr(), self._loss.data_ptr() + 8,
                                             r.V_d.data_ptr(), self._stats.data_ptr(), ws, st))
         allreduce_sum_(self._stats)
         f0, f1 = fractions()
         if row is not None:
-            self._actor_diag(2, r.obs_d, D, r.M, idx, K, actor, r.act_d, r.logp_d, r.rew_d, r.V_d, self._stats.data_ptr(), n, f0, f1,
+            self._actor_diag(2, r.obs_d, D, r.M, idx, K, actor, r.act_d, r.logp_d, rew_d, r.V_d, self._stats.data_ptr(), n, f0, f1,
                              float(self.entropy_coef), row)
             self._step_pair(actor, critic, opti_actor, opti_critic, n, row)
             return
         if self.entropy_coef:
             check(L.mhppo_ppo_grad_ent(D, 2, r.obs_d.data_ptr(), D, r.M, idx, K, r.M, actor.flat.data_ptr(),
-                                       r.act_d.data_ptr(), r.logp_d.data_ptr(), r.rew_d.data_ptr(), r.V_d.data_ptr(), self._stats.data_ptr(),
+                                       r.act_d.data_ptr(), r.logp_d.data_ptr(), rew_d.data_ptr(), r.V_d.data_ptr(), self._stats.data_ptr(),
                                        1.0 / n, f0, f1, float(self.entropy_coef), actor.grad.data_ptr(), self._loss.data_ptr(), ws, st))
             self._step_pair(actor, critic, opti_actor, opti_critic)
             return
         check(L.mhppo_ppo_grad_dev(D, 2, r.obs_d.data_ptr(), D, r.M, idx, K, r.M, actor.flat.data_ptr(),
-                                   r.act_d.data_ptr(), r.logp_d.data_ptr(), r.rew_d.data_ptr(), r.V_d.data_ptr(), self._stats.data_ptr(),
+                                   r.act_d.data_ptr(), r.logp_d.data_ptr(), rew_d.data_ptr(), r.V_d.data_ptr(), self._stats.data_ptr(),
                                    1.0 / n, f0, f1, actor.grad.data_ptr(), self._loss.data_ptr(), ws, st))
         self._step_pair(actor, critic, opti_actor, opti_critic)
 
@@ -425,6 +482,7 @@ class Algo_PPO:
         self.rollout.value_std = self.value_std
         self.rollout._set_head(self.actor_net_cross)
         self.rollout.futur_rewards()                    # also the choice reward rew_d, which GAE mode uses too
+        pending_rn = self._normalize_rewards() if self.normalize_reward else None
         if self.gae_lambda is not None:
             self._prepare_gae()
         clip, sched = self.max_grad_norm is not None, self.lr_schedule
@@ -460,6 +518,11 @@ class Algo_PPO:
             host, done = pending_norms
             done.synchronize()
             self._grad_norms_finish(host.numpy())
+        if pending_rn is not None:
+            host, done = pending_rn
+            done.synchronize()
+            self.last_reward_norm = {k: dict(count=c, mean=m, var=v, scale=math.sqrt(v + 1e-8))
+                                     for k, (c, m, v) in zip(REWARD_STREAMS, host.tolist())}
         if pending_lrs is not None:
             for _, done in pending_lrs:
                 done.synchronize()
@@ -656,6 +719,8 @@ class Algo_PPO:
                 self.ep_grad_norms.append(self.grad_norms_summary())
             if self.lr_schedule is not None:
                 self.ep_lrs.append({p: dict(actor_lr=oa.lr, critic_lr=oc.lr) for p, (oa, oc) in self._pair_optimizers()})
+            if self.normalize_reward:
+                self.ep_reward_norm.append(self.last_reward_norm)
             self.total_loop += 1
             if verbose:
                 print("Episode * {} * cross {:.4f} wait {:.4f} choice {:.4f}  (#cross {} #wait {})".format(

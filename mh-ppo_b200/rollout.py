@@ -47,6 +47,7 @@ class Env_rollout:
         self.use_graph = True                            # replay the T-step loop as a CUDA graph (mhppo_rollout_steps)
         self.value_std = 0.5                             # exploration variance of the Gaussian head (Algo_PPO.value_std, PY:726)
         self.ret = None                                  # GAE returns [S]: allocated by the first gae() call
+        self.rew_n = self.rew_dn = None                  # normalised rewards [S] / [M] (Algo_PPO(normalize_reward=True)), allocated there
 
     def _set_head(self, actor):
         """The kernels' Gaussian head = the actor's own (tanh * std + mean, PY:88-90), the noise variance of PY:726-729 and
@@ -238,20 +239,24 @@ class Env_rollout:
         res["waiting_times"] = wait.permute(2, 0, 1).reshape(-1)          # env-major, like back-to-back episodes of one env
         return res
 
-    def futur_rewards(self):
-        """Expected future rewards (PY:658-684) for every trajectory + the episodic choice reward (PY:461, 504)."""
-        check(self._L.mhppo_returns(self.rew.data_ptr(), self.rl.data_ptr(), self.T, self.M, 0.99, self.rtg.data_ptr(),
+    def futur_rewards(self, rew=None):
+        """Expected future rewards (PY:658-684) for every trajectory + the episodic choice reward (PY:461, 504).  rew: the
+        reward buffer [S] the returns are formed from, self.rew when None (rew_d depends on rl alone)."""
+        rew = self.rew if rew is None else rew
+        check(self._L.mhppo_returns(rew.data_ptr(), self.rl.data_ptr(), self.T, self.M, 0.99, self.rtg.data_ptr(),
                                     self.rew_d.data_ptr(), self._stream()))
         return self.rtg, self.rew_d
 
-    def gae(self, critic_cross, critic_wait, gamma, lam, selections=None, workspace=None):
+    def gae(self, critic_cross, critic_wait, gamma, lam, selections=None, workspace=None, rew=None):
         """GAE(gamma, lambda) returns of the cross / wait buffers, an option of Algo_PPO (the reference's estimator is
         futur_rewards: lambda = 1 against the critic of every epoch).  Each critic evaluates V_old(s) once on the samples
         routed to its net (mhppo_value_stats, into self.V), then one reverse scan per (car, env) column (mhppo_gae) with
         V(s_T) = 0.  selections: the (idx, K) compacted column lists of route 0 and 1 (Algo_PPO._selection), built from
         `route` when None.  Returns (ret [S], stats6): the regression targets and this rank's advantage statistics
-        (sum A, sum A^2, n) of the cross samples, then of the wait samples.  The buffers are allocated on the first call."""
+        (sum A, sum A^2, n) of the cross samples, then of the wait samples.  The buffers are allocated on the first call.
+        rew: the reward buffer [S] to read, self.rew when None."""
         L, st, dev = self._L, self._stream(), self.rew.device
+        rew = self.rew if rew is None else rew
         if self.ret is None:
             self.ret = torch.zeros(self.S, device=dev)
             self._gae_stats = torch.zeros(9, dtype=torch.float64, device=dev)      # stats6 | scratch of mhppo_value_stats
@@ -267,8 +272,8 @@ class Env_rollout:
         ws, scratch = workspace.data_ptr(), self._gae_stats.data_ptr() + 6 * 8
         for critic, (idx, K) in zip((critic_cross, critic_wait), selections):
             check(L.mhppo_value_stats(13, self.obs_c.data_ptr(), 13, self.S, idx.data_ptr(), K, self.M, critic.flat.data_ptr(),
-                                      self.rew.data_ptr(), self.V.data_ptr(), scratch, ws, st))
-        check(L.mhppo_gae(self.rew.data_ptr(), self.V.data_ptr(), self.route.data_ptr(), self.T, self.M, float(gamma), float(lam),
+                                      rew.data_ptr(), self.V.data_ptr(), scratch, ws, st))
+        check(L.mhppo_gae(rew.data_ptr(), self.V.data_ptr(), self.route.data_ptr(), self.T, self.M, float(gamma), float(lam),
                           self.ret.data_ptr(), self._gae_stats.data_ptr(), ws, st))
         return self.ret, self._gae_stats[:6]
 
